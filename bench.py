@@ -2,12 +2,15 @@
 DDIM-50, CFG 7.5) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4]
-                    [--batch-per-gpu B] [--precision bf16|fp32] [--no-cpu-baseline]
+                    [--batch-per-gpu B] [--precision bf16|fp32] [--no-cpu-baseline] [--dump-outputs DIR]
 
 A "step" is one pass of the loop body of models/diffusion.py:223-236 over one batch of synthetic input:
 UNet forward on the CFG-doubled batch + guidance blend + DDIM update.  With N GPUs every rank runs its own
 shard (data parallel, no collective inside a step; one all-gather of the final latents after the timed
 region is checked but not timed).  Rank 0 prints ONE JSON line.  See DESIGN.md §Measurement.
+
+--dump-outputs DIR writes the latents the timed path returned after its last step as DIR/latent.npy (float32;
+inputs and weights are seeded, so two builds run with the same arguments can be compared output for output).
 """
 from __future__ import annotations
 
@@ -40,6 +43,28 @@ CONFIGS = {
     5: dict(arch="sd21", hw=64, steps=1, cfg=False, batch=32, ptype="epsilon", dctx=1024,
             name="SwiftBrush one-step: SD2.1-arch UNet 512^2, ONE forward at t=999, no CFG, batch 256 over 8 GPUs (32 per GPU)"),
 }
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write each tensor as `path/<name>.npy` in float32.  A tensor over its share of DUMP_MAX_BYTES is replaced by a fixed,
+    seeded sample of its flattened elements (same indices in every run of the same shape)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    cap = DUMP_MAX_BYTES // (4 * len(arrays))
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.size > cap:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
+def split_steps(k, regions):
+    """`k` steps as `regions` (at most k) runs of near-equal length."""
+    n = max(1, min(regions, k))
+    return [k // n + (i < k % n) for i in range(n)]
 
 
 def peaks():
@@ -101,7 +126,8 @@ def build_oracle_inputs(cfg, total_batch):
 
 # --------------------------------------------------------------------------------------------------
 def cpu_loop_body_seconds(cfg, sd, arch, hw, n_timed, budget_s):
-    """Seconds per loop-body step of the ORACLE port on the host cores (UNet batch 2B=2 + CFG + DDIM)."""
+    """Seconds per loop-body step of the ORACLE port on the host cores (UNet batch 2B=2 + CFG + DDIM), the number of timed
+    steps, and the latent after the last step."""
     from oracle import sampler_oracle as SO
     from oracle import unet_oracle as UO
     UO.USE_SDPA = True                                     # the reference's stock attention path (models/unet/attention.py:37-43)
@@ -131,7 +157,7 @@ def cpu_loop_body_seconds(cfg, sd, arch, hw, n_timed, budget_s):
             if time.time() - t_start > budget_s and len(times) >= 1:
                 break
     UO.USE_SDPA = False
-    return sum(times) / len(times), len(times)
+    return sum(times) / len(times), len(times), lat
 
 
 def run_reference_arm(args, cfg):
@@ -151,7 +177,9 @@ def run_reference_arm(args, cfg):
         sample = f"loop-body steps on a 32x32 latent, time scaled x{scale:.2f} by algorithmic FLOPs to {cfg['hw']}x{cfg['hw']}"
     torch.set_num_threads(os.cpu_count())
     n = max(1, min(args.steps, int(240 / max(est_full / scale, 0.5))))
-    sec, used = cpu_loop_body_seconds(cfg, sd, arch, hw, n, budget_s=240)
+    sec, used, lat = cpu_loop_body_seconds(cfg, sd, arch, hw, n, budget_s=240)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latent": lat})
     sec *= scale
     img_s = 1.0 / (cfg["steps"] * sec)
     line = {"impl": "reference", "metric": "images_per_sec", "value": img_s, "unit": "images/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -268,6 +296,8 @@ def run_one_step(args, cfg):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms_step = float(t.item()) / K
         finite = bool(torch.isfinite(out).all().item())
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"latent": out})             # rank 0's images: this path has no gather
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -330,8 +360,9 @@ def make_config(cfg, B, ub):
 
 
 def timed_steps(loop, smp, K, Wm, repeats, dev, world, dist, lat_d, ctx_d):
-    """W warm-up steps, then `repeats` regions of EXACTLY K steps each, every region bracketed by barrier + synchronize and
-    timed with CUDA events; per-region time = MAX over ranks.  Returns the sorted per-step times (ms) of the regions."""
+    """W warm-up steps, then EXACTLY K timed steps split into `repeats` regions (at most K), every region bracketed by
+    barrier + synchronize and timed with CUDA events; per-region time = MAX over ranks.  Returns the sorted per-step times
+    (ms) of the regions."""
     n_grid = len(smp.timesteps)
     pos = [0]
 
@@ -350,14 +381,14 @@ def timed_steps(loop, smp, K, Wm, repeats, dev, world, dist, lat_d, ctx_d):
     loop.reset(lat_d, ctx_d)
     run_steps(Wm)
     out = []
-    for _ in range(repeats):
+    for n in split_steps(K, repeats):
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize()
         e0.record()
-        run_steps(K)
+        run_steps(n)
         e1.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -365,16 +396,16 @@ def timed_steps(loop, smp, K, Wm, repeats, dev, world, dist, lat_d, ctx_d):
         t = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        out.append(float(t.item()) / K)
+        out.append(float(t.item()) / n)
     return sorted(out)
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps")
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--repeats", type=int, default=5, help="timed regions of --steps steps each; the median is reported")
+    ap.add_argument("--repeats", type=int, default=5, help="timed regions the --steps steps are split into; the median is reported")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS))
     ap.add_argument("--batch-per-gpu", type=int, default=0)
@@ -386,7 +417,10 @@ def main():
     ap.add_argument("--no-config3", action="store_true", help="N > 1: skip the batch-64-sharded (BASELINE config 3) measurement")
     ap.add_argument("--no-fp32", action="store_true", help="N = 1: skip the one-off fp32-mode ms/step figure")
     ap.add_argument("--no-vae", action="store_true", help="N = 1: skip the VAE-decode (latent -> image) figure")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the latents of the last timed step as DIR/latent.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[args.config])
     if args.batch_per_gpu:
         cfg["batch"] = args.batch_per_gpu
@@ -429,7 +463,8 @@ def main():
         regions = timed_steps(loop, smp, K, Wm, max(1, args.repeats), dev, world, dist, lat_d, ctx_d)
         sampler.stop_flag = True
         ms_step = regions[len(regions) // 2]                  # median region
-        finite = bool(torch.isfinite(loop.latent).all().item())
+        last = loop.latent.clone()                            # the loop state after the last timed step
+        finite = bool(torch.isfinite(last).all().item())
 
         # ---- e2e through the public drop-in API with HOST buffers (UNet.forward + sampler.reverse_process)
         ub = 2 * B if cfg["cfg"] else B
@@ -451,9 +486,8 @@ def main():
 
         for i in range(3):
             e2e_step(i)
-        k2 = max(3, min(K, 20))
         e2e_regions = []
-        for rep in range(max(1, min(args.repeats, 3))):
+        for k2 in split_steps(K, max(1, min(args.repeats, 3))):
             torch.cuda.synchronize()
             if world > 1:
                 dist.barrier()
@@ -496,11 +530,13 @@ def main():
             dist.barrier()
         g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         g0.record()
-        final = gather_latents(loop.latent.clone(), B * world)
+        final = gather_latents(last.clone(), B * world)
         g1.record()
         torch.cuda.synchronize()
         gather_ms = g0.elapsed_time(g1)
         assert final.shape[0] == B * world
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"latent": final})
         launches_per_step = loop.launches_per_step
 
         # ---- N > 1: BASELINE config 3 (batch 64 SHARDED over the N GPUs: strong scaling) in the same run
@@ -606,7 +642,7 @@ def main():
     line = {
         "metric": "images_per_sec", "value": imgs_per_s, "unit": "images/s", "n_gpus": world, "steps": K, "warmup": Wm,
         "ms_per_step": ms_step, "ms_per_step_min": regions[0], "ms_per_step_max": regions[-1], "repeats": len(regions),
-        "timing": "median of `repeats` CUDA-event-timed regions of `steps` steps each (max over ranks per region)",
+        "timing": "`steps` steps split into `repeats` CUDA-event-timed regions; median of the regions' per-step times (max over ranks per region)",
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": args.precision, "data": "synthetic",
         "config": make_config(cfg, B, ub), "cuda_graph": not args.no_graph, "finite": finite,
@@ -615,7 +651,7 @@ def main():
         "e2e": {"value": e2e_imgs, "unit": "images/s", "ms_per_step": e2e_ms, "ms_per_step_min": e2e_regions[0], "ms_per_step_max": e2e_regions[-1],
                 "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                 "api": "UNet.forward + DDIMSampler.reverse_process, pinned host buffers in and out every step"},
-        "gpu_launches": launches_per_step * K * len(regions),
+        "gpu_launches": launches_per_step * K,
         "gather_latents_ms": gather_ms,
         "roofline": roof,
     }
@@ -634,7 +670,7 @@ def main():
             line["torch_eager_same_gpu"] = {"error": repr(ex)}
     if not args.no_cpu_baseline and world >= 1:
         try:
-            sec, used = cpu_loop_body_seconds(cfg, sd, arch, cfg["hw"], 2, budget_s=45)
+            sec, used, _ = cpu_loop_body_seconds(cfg, sd, arch, cfg["hw"], 2, budget_s=45)
             line["cpu_baseline"] = {"value": 1.0 / (cfg["steps"] * sec), "unit": "images/s", "cores": torch.get_num_threads(), "kind": "port",
                                     "sample": f"{used} loop-body steps (after 1 warm-up) of the oracle port (SDPA attention as attention.py:37-43) at {cfg['hw']}x{cfg['hw']}, extrapolated x{cfg['steps']}",
                                     "s_per_step": sec}
