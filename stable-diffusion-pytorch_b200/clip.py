@@ -11,17 +11,14 @@ attention (head_dim 64), out-projection with the residual add in the epilogue, M
 from __future__ import annotations
 
 import json
-import math
 import os
 from dataclasses import dataclass
-from typing import Dict
 
 import torch
 from torch import nn
 
-from . import _lib
-from ._lib import BF16_T, F32_T
-from .unet import _DT, StepProgram, _Node, read_knobs
+from ._lib import F32_T
+from .program import GraphRunner, KernelWeights, LaunchProgram, ProgramModule
 
 
 @dataclass
@@ -81,48 +78,32 @@ _KEYS = {
 }
 
 
-class TextWeights:
+class TextWeights(KernelWeights):
     """Kernel-layout copies of the parameters on one device for one precision (q|k|v fused, GEMM weights k-block-major bf16)."""
 
-    def __init__(self, net, device, precision):
-        with torch.inference_mode(False), torch.no_grad():
-            self.device, self.precision = device, precision
-            wdt = torch.float32 if precision == "fp32" else torch.bfloat16
-            kmajor = precision != "fp32"
-            sd = {k: v.detach() for k, v in net.named_parameters()}
-            K = _KEYS[net.kind]
-            t: Dict[str, torch.Tensor] = {}
-
-            def dev(x, dt=torch.float32):
-                x = x.to(device=device, dtype=dt)
-                if kmajor and dt == torch.bfloat16 and x.dim() == 2 and x.shape[1] % 64 == 0:
-                    n, k = x.shape
-                    x = x.view(n, k // 64, 64).permute(1, 0, 2)
-                return x.contiguous()
-
-            t["tok"], t["pos"] = dev(sd[K["tok"]]), dev(sd[K["pos"]])
-            for i in range(net.layers):
-                p = K["layer"].format(i=i)
-                for j, nm in ((1, K["ln1"]), (2, K["ln2"])):
-                    t[f"{i}.ln{j}.g"], t[f"{i}.ln{j}.b"] = dev(sd[f"{p}.{nm}.weight"]), dev(sd[f"{p}.{nm}.bias"])
-                t[f"{i}.qkv.w"] = dev(torch.cat([sd[f"{p}.self_attn.{n}_proj.weight"] for n in "qkv"], 0), wdt)
-                t[f"{i}.qkv.b"] = dev(torch.cat([sd[f"{p}.self_attn.{n}_proj.bias"] for n in "qkv"], 0))
-                t[f"{i}.o.w"], t[f"{i}.o.b"] = dev(sd[f"{p}.self_attn.out_proj.weight"], wdt), dev(sd[f"{p}.self_attn.out_proj.bias"])
-                t[f"{i}.fc1.w"], t[f"{i}.fc1.b"] = dev(sd[f"{p}.{K['fc1']}.weight"], wdt), dev(sd[f"{p}.{K['fc1']}.bias"])
-                t[f"{i}.fc2.w"], t[f"{i}.fc2.b"] = dev(sd[f"{p}.{K['fc2']}.weight"], wdt), dev(sd[f"{p}.{K['fc2']}.bias"])
-            t["lnf.g"], t["lnf.b"] = dev(sd["final_layer_norm.weight"]), dev(sd["final_layer_norm.bias"])
-            self.t = t
+    def _pack(self, net):
+        sd, t, dev, wdt = self.sd, self.t, self.dev, self.wdt
+        K = _KEYS[net.kind]
+        t["tok"], t["pos"] = dev(sd[K["tok"]]), dev(sd[K["pos"]])
+        for i in range(net.layers):
+            p = K["layer"].format(i=i)
+            for j, nm in ((1, K["ln1"]), (2, K["ln2"])):
+                t[f"{i}.ln{j}.g"], t[f"{i}.ln{j}.b"] = dev(sd[f"{p}.{nm}.weight"]), dev(sd[f"{p}.{nm}.bias"])
+            t[f"{i}.qkv.w"] = dev(torch.cat([sd[f"{p}.self_attn.{n}_proj.weight"] for n in "qkv"], 0), wdt)
+            t[f"{i}.qkv.b"] = dev(torch.cat([sd[f"{p}.self_attn.{n}_proj.bias"] for n in "qkv"], 0))
+            t[f"{i}.o.w"], t[f"{i}.o.b"] = dev(sd[f"{p}.self_attn.out_proj.weight"], wdt), dev(sd[f"{p}.self_attn.out_proj.bias"])
+            t[f"{i}.fc1.w"], t[f"{i}.fc1.b"] = dev(sd[f"{p}.{K['fc1']}.weight"], wdt), dev(sd[f"{p}.{K['fc1']}.bias"])
+            t[f"{i}.fc2.w"], t[f"{i}.fc2.b"] = dev(sd[f"{p}.{K['fc2']}.weight"], wdt), dev(sd[f"{p}.{K['fc2']}.bias"])
+        t["lnf.g"], t["lnf.b"] = dev(sd["final_layer_norm.weight"]), dev(sd["final_layer_norm.bias"])
 
 
-class TextEncoderProgram(StepProgram):
+class TextEncoderProgram(LaunchProgram):
     """One forward for fixed (B, S): openclip.py:133-137 / clip.py:28-34 as a flat launch list."""
 
-    def __init__(self, net, pw: TextWeights, B, S):
-        with torch.inference_mode(False), torch.no_grad(), torch.cuda.device(pw.device):
-            self._init_common(net, pw, B)
-            self._build_text(net, B, S)
+    IO_REGIONS = (("out", "out"), ("ids", "ids_in"))
 
-    def _build_text(self, net, B, S):
+    def _build(self, S):
+        net, B = self.net, self.B
         t, lib = self.pw.t, self.lib
         Cc, heads, inter = net.hidden, net.heads, net.inter
         D, M = Cc // heads, B * S
@@ -154,64 +135,16 @@ class TextEncoderProgram(StepProgram):
         self.out = torch.empty((B, S, Cc), dtype=torch.float32, device=dev)
         self._emit(lib.sdk_layernorm, x.data_ptr(), t["lnf.g"].data_ptr(), t["lnf.b"].data_ptr(), float(net.eps), self.out.data_ptr(), F32_T, M, Cc)
         self.pool.put(x)
-        need = max([int(lib.sdk_tc_gemm_workspace_bytes(hd)) for hd in self.tc_handles] + [0])
-        self.tc_ws = torch.zeros(max(need, 256), dtype=torch.uint8, device=dev)
-        for hd in self.tc_handles:
-            _lib.check(lib.sdk_tc_gemm_set_workspace(hd, self.tc_ws.data_ptr()))
-        self.n_launch = len(self.ops)
 
 
-class _TextBase(nn.Module):
+class _TextBase(ProgramModule):
     """Shared machinery of the two reference text-encoder classes."""
 
     def _setup(self, kind, vocab, hidden, heads, layers, inter, max_len, eps):
         if hidden % heads or hidden // heads not in (40, 64, 80, 160) or hidden % 64:
             raise ValueError(f"hidden_size {hidden} / heads {heads}: head_dim must be 40, 64, 80 or 160 and hidden_size a multiple of 64")
         self.kind, self.vocab, self.hidden, self.heads, self.layers, self.inter, self.max_len, self.eps = kind, vocab, hidden, heads, layers, inter, max_len, eps
-        for name, shape in text_param_spec(kind, vocab, hidden, heads, layers, inter, max_len):
-            self._register(name, shape)
-        read_knobs(self)
-        self._packed: Dict = {}
-        self._plans: Dict = {}
-        self.register_load_state_dict_post_hook(lambda module, incompatible: module.invalidate())
-
-    def _register(self, name, shape):
-        parts = name.split(".")
-        node = self
-        for p in parts[:-1]:
-            if p not in node._modules:
-                node.add_module(p, _Node())
-            node = node._modules[p]
-        leaf = parts[-1]
-        tns = torch.empty(shape)
-        if "norm" in parts[-2]:
-            tns.fill_(1.0 if leaf == "weight" else 0.0)
-        elif "embedding" in parts[-2]:
-            tns.normal_()                                      # nn.Embedding default
-        else:
-            wshape = shape if leaf == "weight" else tuple(getattr(node, "weight").shape)
-            bound = 1.0 / math.sqrt(wshape[1])
-            tns.uniform_(-bound, bound)
-        node.register_parameter(leaf, nn.Parameter(tns, requires_grad=False))
-
-    def invalidate(self):
-        self._packed.clear()
-        self._plans.clear()
-
-    def _apply(self, fn, recurse=True):
-        probe = next(self.parameters())
-        before = (probe.device, probe.dtype, probe.data_ptr())
-        out = super()._apply(fn, recurse)
-        probe = next(self.parameters())
-        if (probe.device, probe.dtype, probe.data_ptr()) != before:
-            self.invalidate()
-        return out
-
-    def set_precision(self, precision: str):
-        if precision not in ("fp32", "bf16"):
-            raise ValueError("precision must be 'fp32' or 'bf16'")
-        self.precision = precision
-        return self
+        self._init_params(text_param_spec(kind, vocab, hidden, heads, layers, inter, max_len))
 
     def gradient_checkpointing_enabled(self, enabled=False):       # reference API no-ops (clip.py:19-27)
         return None
@@ -235,8 +168,10 @@ class _TextBase(nn.Module):
         pkey = key + (B, S)
         run = self._plans.get(pkey)
         if run is None:
-            run = self._plans[pkey] = _TextRunner(TextEncoderProgram(self, pw, B, S), self.use_cuda_graph)
-        return run(x)
+            run = self._plans[pkey] = GraphRunner(TextEncoderProgram(self, pw, B, S), self.use_cuda_graph)
+        run.prog.ids_in.copy_(x.to(torch.int64), non_blocking=True)
+        run.run()
+        return run.prog.out.clone()
 
 
 class CLIPTextModel(_TextBase):
@@ -284,27 +219,3 @@ class OpenCLIP(nn.Module):
     def encode_text(self, input_ids: torch.Tensor) -> torch.Tensor:
         return self.text_model(input_ids)
 
-
-class _TextRunner:
-    def __init__(self, prog: TextEncoderProgram, use_graph: bool):
-        self.prog, self.use_graph, self.graph, self.calls = prog, use_graph, None, 0
-
-    def __call__(self, ids):
-        p = self.prog
-        p.ids_in.copy_(ids.to(torch.int64), non_blocking=True)
-        self.calls += 1
-        with torch.cuda.device(p.device):
-            if not self.use_graph:
-                p.launch(p.ops)
-            elif self.graph is None:
-                if self.calls == 1:
-                    p.launch(p.ops)
-                else:
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        p.launch(p.ops)
-                    self.graph = g
-                    g.replay()
-            else:
-                self.graph.replay()
-        return p.out.clone()

@@ -19,6 +19,7 @@ from typing import Optional
 import torch
 
 from . import _lib
+from .program import GraphRunner
 from .scheduler import PRED_EPS, PRED_V, DDIMSampler, DDPMSampler, x0_from_eps
 from .unet import StepProgram, UNet, same_context, tensor_version
 
@@ -46,8 +47,7 @@ class DenoiseLoop:
         self.lib = _lib.lib()
         pw = unet._weights(self.device)
         self.prog = StepProgram(unet, pw, ub, height, width, 1, bc, context_len, b_src=batch)
-        self.use_graph = unet.use_cuda_graph if use_cuda_graph is None else use_cuda_graph
-        self.graph = None
+        self.runner = GraphRunner(self.prog, unet.use_cuda_graph if use_cuda_graph is None else use_cuda_graph, self._enqueue_step)
         self.latent = self.prog.x_in                         # the loop state IS the UNet's input staging buffer
         with torch.inference_mode(False), torch.no_grad():     # loop state stays writable when built under inference_mode
             self.noise = torch.empty_like(self.latent) if isinstance(sampler, DDPMSampler) else None
@@ -73,7 +73,7 @@ class DenoiseLoop:
                 raise RuntimeError(f"mask must hold one value per latent pixel ({self.H}x{self.W})")
             self.inpaint_orig = o
             self.inpaint_mask = mask.to(self.device).reshape(self.H * self.W).ne(0).to(torch.uint8).contiguous()
-        self.graph = None                                      # pointers are baked into the captured launches
+        self.runner.graph = None                               # pointers are baked into the captured launches
 
     # ---- one step = [next timestep] + UNet program + [CFG + scheduler update in place] -------------------
     def _enqueue_step(self):
@@ -159,7 +159,7 @@ class DenoiseLoop:
             self.ts_table = s.timesteps.to(self.device, torch.int64).contiguous()
             self.coef = s._coef_table(self.device, 0.0)
             self._grid_key = key
-            self.graph = None                                  # tables are baked into the captured launches
+            self.runner.graph = None                           # tables are baked into the captured launches
             # time embedding -> 22 ResBlock projections depend only on t: run that chain once per grid point, keep the rows
             self.tb_table = None
             if self.hoist_time and p.nt == 1:
@@ -181,21 +181,7 @@ class DenoiseLoop:
         if isinstance(self.sampler, DDPMSampler):
             # same global-RNG draw as ddpm.py:80, outside the graph so torch's generator state advances normally
             self.noise.copy_(torch.randn(self.latent.shape, dtype=self.latent.dtype, device=self.device))
-        with torch.cuda.device(self.device):
-            if not self.use_graph:
-                self._enqueue_step()
-            elif self.graph is None:
-                if not getattr(self, "_warm", False):
-                    self._enqueue_step()
-                    self._warm = True
-                else:
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        self._enqueue_step()
-                    self.graph = g
-                    g.replay()
-            else:
-                self.graph.replay()
+        self.runner.run()
 
     def reset(self, latent: torch.Tensor, context: torch.Tensor):
         if tuple(latent.shape) != tuple(self.latent.shape):

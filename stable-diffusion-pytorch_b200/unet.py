@@ -15,21 +15,15 @@ Precision modes (``net.precision``):
 """
 from __future__ import annotations
 
-import ctypes as C
 import json
-import math
 import os
-import struct
 from typing import Dict, List, Optional, Union
 
 import torch
-from torch import nn
 
-from . import _lib
-from ._lib import BF16_T, F32_T, AttentionTcDesc, ConvParams, LinearLnDesc, TcGemmDesc
-from .arch import BLOCK_OUT, Conv, ResBlock, Transformer, UNetArch, build_arch, param_spec
-
-_DT = {F32_T: torch.float32, BF16_T: torch.bfloat16}
+from ._lib import BF16_T, F32_T
+from .arch import BLOCK_OUT, Transformer, UNetArch, build_arch, param_spec
+from .program import _DT, GraphRunner, KernelWeights, LaunchProgram, ProgramModule
 
 
 def tensor_version(t: torch.Tensor):
@@ -48,43 +42,10 @@ def same_context(cond: torch.Tensor, ref, version) -> bool:
     return cond is ref and v is not None and v == version
 
 
-def read_knobs(m):
-    """Environment knobs of the launch-list programs (DESIGN.md 7a); defaults are the measured best on B200."""
-    m.precision = os.environ.get("SDB200_PRECISION", "bf16")
-    m.tc_block_n = int(os.environ.get("SDB200_TC_BLOCK_N", "0"))      # 0 = auto; tuning / test overrides
-    m.tc_splits = int(os.environ.get("SDB200_TC_SPLITS", "0"))
-    m.tc_tune_pairs = int(os.environ.get("SDB200_TC_TUNE_PAIRS", "0"))   # also try cta_group::2 pairs when measuring tilings
-    m.tc_autotune = int(os.environ.get("SDB200_TC_AUTOTUNE", "1"))     # 0 model | 1 committed cache | 2 measure misses | 3 and print
-    m.attn_tc = os.environ.get("SDB200_ATTN_TC", "1") != "0"          # tcgen05 attention (head_dim 40 / 64 / 80 / 160); 0: mma.sync kernel
-    # bf16: LayerNorm folded into the consuming GEMM (built and parity-tested; measured on B200 it costs the GEMMs 0.23 ms per step and
-    # saves 0.20 ms of layernorm launches at UNet batch 2, and loses 0.9 ms of 20.3 at batch 16 -> opt-in)
-    m.ln_fold = os.environ.get("SDB200_LN_FOLD", "0") != "0"
-    # bf16: projection (+ bias + residual) and the LayerNorm of its output rows in ONE cluster launch (linear_ln.cu) for layers
-    # whose grid fits one wave of the chip -- the latency-bound case (every transformer layer at UNet batch 2)
-    m.ln_fuse = os.environ.get("SDB200_LN_FUSE", "1") != "0"
-    m.ln_fuse_max_ctas = int(os.environ.get("SDB200_LN_FUSE_MAX_CTAS", "0"))      # 0 = the SM count of the device (one wave)
-    m.fold_gathers = os.environ.get("SDB200_FOLD_GATHERS", "1") != "0"   # bf16: stride-2 / upsample gathers inside the GEMM's TMA coordinates
-    # ... where the layer has enough rows to fill the chip WITHOUT split-K (the folded form runs on the persistent kernel only; measured
-    # on B200 at UNet batch 2: the 8x8 / 16x16 layers are weight-streaming bound and 1.6-3x faster as im2col / upsample + split-K GEMM)
-    m.fold_min_rows_up = int(os.environ.get("SDB200_FOLD_MIN_ROWS_UP", "512"))      # low-res rows B*h*w of an upsample conv
-    m.fold_min_rows_s2 = int(os.environ.get("SDB200_FOLD_MIN_ROWS_S2", "2048"))     # output rows of a stride-2 conv
-    m.ln_fold_min_rows = int(os.environ.get("SDB200_LN_FOLD_MIN_ROWS", "0"))   # ... only for token counts >= this (small ones are split-K GEMMs)
-    m.tc_two_cta = int(os.environ.get("SDB200_TC_TWO_CTA", "0"))       # 0 auto, 1 never, 2 always (even m-tiles)
-    # sums: statistics from per-channel sums reduced in the producing GEMM's epilogue (bf16 program; fastest measured) |
-    # split (stats + apply kernels) | cluster | coop | auto
-    m.gn_mode = os.environ.get("SDB200_GN_MODE", "sums")
-    m.gn_cluster_max_bytes = int(os.environ.get("SDB200_GN_CLUSTER_MAX_BYTES", str(3 << 20)))
-    m.use_cuda_graph = os.environ.get("SDB200_CUDA_GRAPH", "1") != "0"
-
-
-class _Node(nn.Module):
-    """Anonymous container so parameters get the reference's dotted names."""
-
-
 # ======================================================================================
 # weight packing
 # ======================================================================================
-class PackedWeights:
+class PackedWeights(KernelWeights):
     """Kernel-layout copies of the parameters on one device for one precision.
 
     conv  [N][Cin][kh][kw] -> [N][kh][kw][Cin]   (K-major rows, NHWC gather order)
@@ -94,49 +55,17 @@ class PackedWeights:
     t_embed of all 22 ResBlocks -> one [sum Cout][1280] matrix (single batched mat-vec)
     """
 
-    def __init__(self, net: "UNet", device, precision: str):
-        # normal (non-inference) tensors even when the first forward runs under torch.inference_mode()
-        with torch.inference_mode(False), torch.no_grad():
-            self._pack(net, device, precision)
-
-    def _pack(self, net: "UNet", device, precision: str):
-        self.device, self.precision = device, precision
-        wdt = torch.float32 if precision == "fp32" else torch.bfloat16
-        self.wcode = F32_T if precision == "fp32" else BF16_T
-        a = net.arch
-        sd = {k: v.detach() for k, v in net.named_parameters()}
-        t: Dict[str, torch.Tensor] = {}
-
-        kmajor = precision != "fp32"
-
-        def dev(x, dt=torch.float32):
-            x = x.to(device=device, dtype=dt)
-            if kmajor and dt == torch.bfloat16 and x.dim() == 2 and x.shape[1] % 64 == 0:
-                # tensor-core operand: k-block-major [K/64][N][64] -> every B stage is one contiguous run of HBM
-                n, k = x.shape
-                x = x.view(n, k // 64, 64).permute(1, 0, 2)
-            return x.contiguous()
-
-        def conv_w(name, dt=wdt):
-            w = sd[name]                                  # [N, Cin, kh, kw]
-            return dev(w.permute(0, 2, 3, 1).reshape(w.shape[0], -1), dt)
-
+    def _pack(self, net: "UNet"):
+        a, sd, t, wdt, dev, conv_w = net.arch, self.sd, self.t, self.wdt, self.dev, self.conv_w
+        device, precision = self.device, self.precision
         for k in ("time_embedding.ffn.0.weight", "time_embedding.ffn.0.bias",
                   "time_embedding.ffn.2.weight", "time_embedding.ffn.2.bias"):
             t[k] = dev(sd[k])
         t["tb.w"] = torch.cat([sd[f"{r.prefix}.t_embed.weight"] for r in a.res_blocks], 0).to(device=device, dtype=wdt).contiguous()
         t["tb.b"] = dev(torch.cat([sd[f"{r.prefix}.t_embed.bias"] for r in a.res_blocks], 0))
-        t["conv_in.w"] = conv_w("encoder.conv_in.weight", torch.float32)
-        t["conv_in.b"] = dev(sd["encoder.conv_in.bias"])
+        self.conv_in("encoder.conv_in")
         for r in a.res_blocks:
-            p = r.prefix
-            for n in ("groupnorm_1", "groupnorm_2"):
-                t[f"{p}.{n}.g"], t[f"{p}.{n}.b"] = dev(sd[f"{p}.{n}.weight"]), dev(sd[f"{p}.{n}.bias"])
-            for n in ("conv_1", "conv_2"):
-                t[f"{p}.{n}.w"], t[f"{p}.{n}.b"] = conv_w(f"{p}.{n}.weight"), dev(sd[f"{p}.{n}.bias"])
-            if r.has_proj:
-                t[f"{p}.proj.w"], t[f"{p}.proj.b"] = conv_w(f"{p}.proj_input.weight"), dev(sd[f"{p}.proj_input.bias"])
-                t[f"{p}.conv2_proj.b"] = dev(sd[f"{p}.conv_2.bias"].float() + sd[f"{p}.proj_input.bias"].float())
+            self.res_block(r.prefix, ("groupnorm_1", "groupnorm_2"), ("conv_1", "conv_2"), "proj_input")
         kv_list = []
         for tr in a.transformers:
             p, b, c = tr.prefix, f"{tr.prefix}.transformer_block", tr.c
@@ -174,26 +103,13 @@ class PackedWeights:
             if precision != "fp32" and getattr(net, "ln_fold", False):
                 fold("ff0", torch.stack([w0[:4 * c], w0[4 * c:]], 1).reshape(8 * c, c), torch.stack([b0[:4 * c], b0[4 * c:]], 1).reshape(8 * c), 3)
             t[f"{p}.ff1.w"], t[f"{p}.ff1.b"] = dev(sd[f"{b}.ffn.1.weight"], wdt), dev(sd[f"{b}.ffn.1.bias"])
-        for st in a.down + a.up:
+        for st in a.down:
             if st.resample is not None:
                 p = st.resample.prefix
                 t[f"{p}.w"], t[f"{p}.b"] = conv_w(f"{p}.weight"), dev(sd[f"{p}.bias"])
-                if precision != "fp32" and st in a.up:
-                    # nearest-2x upsample + 3x3 conv (unet.py:248-251) == four 2x2 convs on the low-res input, one per output
-                    # parity: the 3x3 taps that land on the same input pixel are summed (fp32) before the bf16 rounding
-                    w = sd[f"{p}.weight"].to(device=device, dtype=torch.float32).permute(0, 2, 3, 1)          # [N][kh][kw][C]
-                    rows = {0: ([0], [1, 2]), 1: ([0, 1], [2])}
-                    sets = []
-                    for py in (0, 1):
-                        for px in (0, 1):
-                            wp = torch.zeros((w.shape[0], 2, 2, w.shape[3]), dtype=torch.float32, device=device)
-                            for ia in (0, 1):
-                                for ib in (0, 1):
-                                    for kh in rows[py][ia]:
-                                        for kw in rows[px][ib]:
-                                            wp[:, ia, ib] += w[:, kh, kw]
-                            sets.append(dev(wp.reshape(w.shape[0], -1), torch.bfloat16))                      # k-block-major [4C/64][N][64]
-                    t[f"{p}.w_up2"] = torch.cat(sets, 0).contiguous()
+        for st in a.up:
+            if st.resample is not None:
+                self.upsample_conv(st.resample.prefix)
         # cross-attention K/V projections of every transformer, rows concatenated: the context program is one [Bc*77, dctx] x
         # [sum 2C, dctx]^T GEMM (24960 output columns for SD1.5) instead of 16 launches; kv_off[index] = first column of a layer
         self.kv_off, self.kv_total = {}, 0
@@ -204,50 +120,18 @@ class PackedWeights:
             t["kv2_all.w"] = dev(torch.cat([w for _, w in kv_list], 0), wdt)
         t["out.gn.g"], t["out.gn.b"] = dev(sd["output.0.weight"]), dev(sd["output.0.bias"])
         t["out.w"], t["out.b"] = conv_w("output.2.weight", wdt), dev(sd["output.2.bias"])
-        self.t = t
-
-    def ptr(self, name) -> int:
-        return self.t[name].data_ptr()
 
 
 # ======================================================================================
 # step program
 # ======================================================================================
-class _Pool:
-    """Activation pool with explicit liveness: buffers are handed out and returned at plan time, so
-    the program's peak footprint is the max live set, not the sum of all intermediates."""
+class StepProgram(LaunchProgram):
+    """One UNet forward for fixed (B, H, W, n_timesteps, cond batch, Sk) as a flat launch list.  ``time_ops`` is its time-embedding
+    chain (timestep -> self.tb) and ``body_ops`` the forward without it."""
 
-    def __init__(self, device):
-        self.device = device
-        self.free: Dict[int, List[torch.Tensor]] = {}
-        self.all: List[torch.Tensor] = []
-        self.owner: Dict[int, torch.Tensor] = {}
-
-    def get(self, rows: int, cols: int, code: int) -> torch.Tensor:
-        dt = _DT[code]
-        nbytes = rows * cols * (4 if code == F32_T else 2)
-        nbytes = (nbytes + 255) // 256 * 256
-        lst = self.free.get(nbytes)
-        raw = lst.pop() if lst else None
-        if raw is None:
-            raw = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-            self.all.append(raw)
-        v = raw[: rows * cols * (4 if code == F32_T else 2)].view(dt).view(rows, cols)
-        self.owner[id(v)] = raw
-        v._pool_raw = raw
-        return v
-
-    def put(self, v: torch.Tensor):
-        raw = self.owner.pop(id(v))
-        self.free.setdefault(raw.numel(), []).append(raw)
-
-    @property
-    def nbytes(self):
-        return sum(r.numel() for r in self.all)
-
-
-class StepProgram:
-    """One UNet forward for fixed (B, H, W, n_timesteps, cond batch, Sk) as a flat launch list."""
+    PROGRAM_IDS = {"ops": 0, "ctx_ops": 1, "time_ops": 2, "body_ops": 3}
+    PROGRAM_LOOP_STEP = 4                   # one sampler step of DenoiseLoop.export_engine
+    IO_REGIONS = (("x", "x_in"), ("timestep", "t_in"), ("context", "cond_in"), ("out", "out"))
 
     def __init__(self, net: "UNet", pw: PackedWeights, B, H, W, nt, Bc, Sk, b_src=None):
         if Bc not in (1, B):
@@ -255,460 +139,147 @@ class StepProgram:
             raise RuntimeError(f"context batch {Bc} neither matches nor broadcasts to the UNet batch {B}")
         if nt not in (1, B):
             raise RuntimeError(f"timestep count {nt} neither matches nor broadcasts to the UNet batch {B}")
-        # buffers are ordinary tensors (a plan built under torch.inference_mode() must stay writable afterwards) and every
-        # launch / allocation happens with the plan's device current (handles cache per-device state)
-        with torch.inference_mode(False), torch.no_grad(), torch.cuda.device(pw.device):
-            self._plan(net, pw, B, H, W, nt, Bc, Sk, b_src)
+        super().__init__(net, pw, B, H, W, nt, Bc, Sk, b_src)
 
-    def _init_common(self, net, pw, B):
-        """State shared by every launch-list program built from these emit helpers (UNet step, VAE decoder, text encoder)."""
-        self.net, self.pw, self.B = net, pw, B
-        dev = pw.device
-        self.device = dev
-        self.precision = pw.precision
-        self.act = F32_T if pw.precision == "fp32" else BF16_T       # GEMM operand type
-        self.lib = _lib.lib()
-        self.ops = []            # main program: [(fn, args)]
-        self.ctx_ops = []        # context program (cross-attention K/V), re-run only when cond changes
-        self.keep = []           # ctypes structs / tensors that must outlive the launches
-        self.pool = _Pool(dev)
-        self.n_launch = 0
-        self.tc_handles = []
-        self.attn_handles = []
-        self.lln_handles = []
-        self._handle_meta = []   # (kind, handle, descriptor, aux) of every tensor-core handle: what the plan-level C entry adopts
-        self.consts = []         # constant device tensors created by the planner itself (beside the packed weights)
-        self.plan = None         # sdk_plan (built on first launch): the launch lists behind the C ABI
-        self._plan_ids = {}
-        # GroupNorm statistics from per-channel sums accumulated by the producing GEMM (bf16 program) instead of a statistics
-        # kernel.  All tables live in one arena that the program zeroes with its first op.
-        self.gn_from_sums = pw.precision != "fp32" and net.gn_mode == "sums"
-        self.stat_arena = torch.zeros(max(4, 2 * B) << 20, dtype=torch.uint8, device=dev) if self.gn_from_sums else None
-        self.stat_used = 0
-
-    def _plan(self, net, pw, B, H, W, nt, Bc, Sk, b_src):
-        self._init_common(net, pw, B)
-        self.b_src = B if b_src is None else b_src     # latent rows actually stored: B == 2*b_src folds latent.repeat(2,...)
+    def _build(self, H, W, nt, Bc, Sk, b_src):
+        self.b_src = self.B if b_src is None else b_src    # latent rows actually stored: B == 2*b_src folds latent.repeat(2,...)
         self.H, self.W, self.nt, self.Bc, self.Sk = H, W, nt, Bc, Sk
-        a: UNetArch = net.arch
+        a: UNetArch = self.net.arch
         self.arch = a
-        dev = pw.device
-
-        f32 = torch.float32
+        t, lib = self.pw.t, self.lib
+        B = self.B
+        dev, f32 = self.device, torch.float32
         # static I/O staging (graph-stable addresses)
         self.x_in = torch.empty((self.b_src, a.in_channels, H, W), dtype=f32, device=dev)
         self.t_in = torch.zeros((nt,), dtype=torch.int64, device=dev)
         self.cond_in = torch.empty((Bc, Sk, a.dctx), dtype=f32, device=dev)
         self.out = torch.empty((B, a.out_channels, H, W), dtype=f32, device=dev)
-        self.gn_ws = torch.zeros(int(self.lib.sdk_groupnorm_workspace_bytes(B, H * W)), dtype=torch.uint8, device=dev)
+        self.gn_ws = torch.zeros(int(lib.sdk_groupnorm_workspace_bytes(B, H * W)), dtype=torch.uint8, device=dev)
         self.gn_stats = torch.empty((B, 32, 2), dtype=f32, device=dev)
         self.kv: Dict[int, torch.Tensor] = {}
-        self._build()
-
-    # ---- emit helpers -----------------------------------------------------------------
-    def _emit(self, fn, *args, ctx=False):
-        (self.ctx_ops if ctx else self.ops).append((fn, args))
-
-    def _conv(self, srcs, w, bias, B, Hin, Win, N, *, k=1, stride=1, up=False, tbias=0, tb_stride=0,
-              residual=None, geglu=False, out_code=F32_T, out=None, out_nchw=False, in_code=None, ctx=False,
-              force_simt=False, seg2=None, want_stats=False, ln_out=False, ln_in=None, fold_gather=False, w_rowmajor=False):
-        """srcs: [(tensor[rows, C], C)] (1 or 2).  Returns the output tensor [M, N or N/2].
-        w_rowmajor: ``w`` is a plain [N][K] matrix (an ACTIVATION used as the B operand: attention scores, P V) instead of packed weights.
-        want_stats: the output feeds a GroupNorm -> also produce its per-channel (sum, sum of squares) table (out._cstats).
-        ln_out: the output feeds a LayerNorm that is folded into its consumer -> also produce a bf16 copy (out._bf16) and the per-row
-        statistics partials (out._rowstats).  ln_in = (row statistics tensor, column sums of the folded weights): this GEMM applies
-        the LayerNorm of its A rows in its epilogue (tensor-core path only)."""
-        upf = 2 if up else 1
-        pad = k // 2
-        Hout = (Hin * upf + 2 * pad - k) // stride + 1
-        Wout = (Win * upf + 2 * pad - k) // stride + 1
-        M = B * Hout * Wout
-        n_out = N // 2 if geglu else N
-        if out is None:
-            out = self.pool.get(M, n_out, out_code)
-        p = ConvParams()
-        p.src0 = srcs[0][0].data_ptr()
-        p.C0 = srcs[0][1]
-        p.src1 = srcs[1][0].data_ptr() if len(srcs) > 1 else 0
-        p.C1 = srcs[1][1] if len(srcs) > 1 else 0
-        p.weight, p.bias = w.data_ptr(), (bias.data_ptr() if bias is not None else 0)
-        p.tbias, p.tb_stride = tbias, tb_stride
-        p.residual = residual.data_ptr() if residual is not None else 0
-        p.out = out.data_ptr()
-        p.B, p.Hin, p.Win, p.Hout, p.Wout = B, Hin, Win, Hout, Wout
-        p.ksize, p.stride, p.upsample, p.N = k, stride, int(up), N
-        p.in_dtype = self.act if in_code is None else in_code
-        p.out_dtype, p.out_nchw, p.geglu = out_code, int(out_nchw), int(geglu)
-        self.keep.append(p)
-        want_stats = want_stats and self.gn_from_sums and out_code == F32_T and not geglu and not out_nchw
-        cs = self._stat_table(B, N) if want_stats else None
-        fused = False
-        if p.in_dtype == F32_T or force_simt:
-            self._emit(self.lib.sdk_conv_gemm_f32, C.byref(p), ctx=ctx)
-        else:
-            extras = None
-            if ln_out:
-                out._bf16 = self.pool.get(M, N, BF16_T)
-                out._rowstats = self.pool.get(M, 2 * (N // 32), F32_T)
-                extras = dict(out2=out._bf16, row_stats=out._rowstats)
-            if ln_in is not None:
-                extras = dict(extras or {}, ln_stats=ln_in[0], ln_colsum=ln_in[1], ln_parts=srcs[0][1] // 32)
-            if fold_gather:
-                extras = dict(extras or {}, gather="up2" if up else "s2")
-            if w_rowmajor:
-                extras = dict(extras or {}, w_rowmajor=True)
-            fused = self._emit_tc_conv(p, srcs, w, ctx, seg2, cs, extras)
-            if fused is None:                               # folded gather not available for this shape: nothing was emitted
-                self.pool.put(out)
-                return None, Hout, Wout
-        if want_stats:
-            if not fused:                                   # producer cannot reduce its own columns: one extra small launch
-                self._emit(self.lib.sdk_channel_stats, out.data_ptr(), B, Hout * Wout, N, cs.data_ptr(), ctx=ctx)
-            out._cstats = cs
-        return out, Hout, Wout
-
-    def _stat_table(self, B, N):
-        """double [B][N][2] per-channel (sum, sum of squares) table carved from the arena."""
-        nbytes = (B * N * 16 + 255) // 256 * 256
-        if self.stat_used + nbytes > self.stat_arena.numel():
-            raise RuntimeError("statistics arena exhausted")
-        t = self.stat_arena[self.stat_used: self.stat_used + B * N * 16].view(torch.float64).view(B, N, 2)
-        self.stat_used += nbytes
-        return t
-
-    def _emit_tc_conv(self, p, srcs, w, ctx, seg2=None, cs=None, extras=None):
-        """tcgen05 implicit GEMM for a stride-1 conv / linear described by ConvParams ``p``."""
-        gather = (extras or {}).get("gather")
-        if len(srcs) != 1 or ((p.stride != 1 or p.upsample) and not gather):
-            raise RuntimeError("tensor-core conv takes one pre-concatenated bf16 source (stride 2 / upsample only as folded gathers)")
-        d = TcGemmDesc()
-        d.a[0], d.w[0], d.C[0], d.ksize[0], d.nseg = p.src0, p.weight, p.C0, p.ksize, 1
-        if seg2 is not None:                                   # (activation [rows, C2] bf16, C2, 1x1 weights)
-            d.a[1], d.C[1], d.w[1], d.ksize[1], d.nseg = seg2[0].data_ptr(), seg2[1], seg2[2].data_ptr(), 1, 2
-        d.B, d.H, d.W, d.N = p.B, p.Hin, p.Win, p.N
-        if gather == "s2":                                     # stride-2 conv: tiles walk the OUTPUT image, the A box the input
-            d.H, d.W, d.a_stride, d.a_h, d.a_w = p.Hout, p.Wout, 2, p.Hin, p.Win
-        elif gather == "up2":                                  # folded upsample: tiles walk the low-res input, four parities
-            d.up2 = 1
-        d.bias, d.tbias, d.tb_stride, d.residual, d.out = p.bias, p.tbias, p.tb_stride, p.residual, p.out
-        d.out_dtype, d.geglu, d.out_nchw = p.out_dtype, p.geglu, p.out_nchw
-        d.block_n, d.splits, d.w_kmajor, d.two_cta = self.net.tc_block_n, self.net.tc_splits, 1, self.net.tc_two_cta
-        d.w_const = 1                                          # packed weights: constants of the stream (early fetch under PDL)
-        if extras and extras.get("w_rowmajor"):
-            d.w_kmajor, d.w_const = 0, 0                       # the B operand is an activation written by the preceding kernels
-        if extras:
-            if "out2" in extras:
-                d.out2, d.row_stats = extras["out2"].data_ptr(), extras["row_stats"].data_ptr()
-            if "ln_stats" in extras:
-                d.ln_stats, d.ln_colsum = extras["ln_stats"].data_ptr(), extras["ln_colsum"].data_ptr()
-                d.ln_parts, d.ln_eps = extras["ln_parts"], 1e-5
-        if self.net.tc_autotune and not d.block_n and not d.splits:
-            d.block_n, d.splits, d.two_cta = self._autotune(d, srcs[0][0], cs)
-        h = C.c_void_p()
-        rc = self.lib.sdk_tc_gemm_create(C.byref(d), C.byref(h))
-        if rc == -3 and gather:
-            return None                                         # caller falls back to the materialised gather
-        if rc == -3 and extras and ("out2" in extras or "ln_stats" in extras):
-            # the tuned tiling cannot carry the fused LayerNorm work (ragged N tile, or a split-K grid too large to reduce inside the
-            # kernel): an exact N tile without split-K always can
-            d.splits, d.two_cta = 1, 1
-            if d.N % max(d.block_n, 1) != 0:
-                d.block_n = 0
-            rc = self.lib.sdk_tc_gemm_create(C.byref(d), C.byref(h))
-        _lib.check(rc)
-        self.tc_handles.append(h)
-        self.keep.append(d)
-        self._handle_meta.append([1, h, d, cs.data_ptr() if cs is not None else 0])
-        self._emit(self.lib.sdk_tc_gemm_launch, h, ctx=ctx)
-        if cs is None:
-            return False
-        # statistics of the output accumulated by the GEMM's own epilogue into the (zeroed once per step) table
-        rc = self.lib.sdk_tc_gemm_set_stats(h, cs.data_ptr())
-        if rc == -3:                                        # SDK_ERR_UNSUPPORTED: tiling cannot attribute rows to samples
-            self._handle_meta[-1][3] = 0
-            return False
-        _lib.check(rc)
-        return True
-
-    # ---- GEMM tilings: committed measurements (read-only) + optional plan-time measurement -----------------
-    # SDB200_TC_AUTOTUNE = 0: the library's cost model only
-    #                      1: (default) tilings measured on B200 and COMMITTED with the package (tune_cache.json, never written
-    #                         at run time) for the benchmark configurations; the deterministic cost model on a miss
-    #                      2: additionally MEASURE shapes that miss (cold weights, warm activations) and merge them, under a
-    #                         file lock, into the per-user cache SDB200_TC_TUNE_FILE (default ~/.cache/sdb200/tune_cache.json).
-    # A measured tiling changes block_n / split-K and therefore the fp32 summation order: results of two machines with
-    # different user caches agree to rounding, not bit for bit; modes 0/1 are reproducible everywhere.
-    _tune_cache: Dict[str, tuple] = {}
-    _tune_shipped = os.path.join(os.path.dirname(os.path.abspath(__file__)), "tune_cache.json")
-    _tune_loaded = False
-
-    @staticmethod
-    def _tune_user_file():
-        return os.environ.get("SDB200_TC_TUNE_FILE") or os.path.join(os.path.expanduser("~"), ".cache", "sdb200", "tune_cache.json")
-
-    @classmethod
-    def _tune_load(cls):
-        if cls._tune_loaded:
-            return
-        cls._tune_loaded = True
-        paths = (cls._tune_shipped, cls._tune_user_file())
-        if os.environ.get("SDB200_TC_TUNE_IGNORE_SHIPPED", "0") == "1":   # re-measuring after a kernel change
-            paths = paths[1:]
-        for path in paths:                                          # the user's own measurements win
-            try:
-                with open(path) as f:
-                    cls._tune_cache.update({k: tuple(v) for k, v in json.load(f).items()})
-            except (OSError, ValueError):
-                pass
-
-    @classmethod
-    def _tune_save(cls, key, value):
-        """Merge ONE new measurement into the per-user cache (never the package directory); concurrent ranks serialise on a
-        lock file and re-read before writing, so nobody's entries are lost."""
-        path = cls._tune_user_file()
-        try:
-            import fcntl
-            os.makedirs(os.path.dirname(path) or ".", exist_ok=True)
-            with open(path + ".lock", "w") as lk:
-                fcntl.flock(lk, fcntl.LOCK_EX)
-                cur = {}
-                try:
-                    with open(path) as f:
-                        cur = json.load(f)
-                except (OSError, ValueError):
-                    pass
-                cur[key] = list(value)
-                tmp = path + f".{os.getpid()}.tmp"
-                with open(tmp, "w") as f:
-                    json.dump(dict(sorted(cur.items())), f, indent=0)
-                os.replace(tmp, path)
-        except OSError:
-            pass                                             # unwritable home: keep the in-process cache only
-
-    def _autotune(self, d, a_tensor, cs):
-        """Time the candidate (block_n, split-K) tilings of this layer shape on the device, in the state the step sees them:
-        weights cold (each step streams 1.7 GB of them through a 126 MB L2), activations warm.  The library's cost model picks
-        the starting point; this replaces modelled by measured time.  One measurement per distinct shape per process."""
-        StepProgram._tune_load()
-        key = "|".join(str(x) for x in (torch.cuda.get_device_name(self.device), d.B, d.H, d.W, d.N, d.nseg, d.C[0], d.ksize[0], d.C[1],
-                                        d.geglu, d.out_dtype, int(bool(d.residual)), int(bool(d.tbias)), int(cs is not None)))
-        if d.out2 or d.ln_stats:                              # fused LayerNorm work changes the epilogue: its own measurements
-            key += f"|ln{int(bool(d.out2))}{int(bool(d.ln_stats))}"
-        if d.up2 or d.a_stride == 2:
-            key += f"|g{'u' if d.up2 else 's'}"
-        hit = StepProgram._tune_cache.get(key)
-        if hit is not None:
-            return tuple(hit) if len(hit) == 3 else (hit[0], hit[1], d.two_cta)
-        if self.net.tc_autotune < 2:
-            return (0, 0, d.two_cta)                           # miss: deterministic cost model, no measurement, no file written
-        lib = self.lib
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        if not hasattr(self, "_tune_flush"):
-            self._tune_flush = torch.empty(192 << 20, dtype=torch.uint8, device=self.device)
-        total_kb = (d.C[0] // 64) * d.ksize[0] * d.ksize[0] + ((d.C[1] // 64) if d.nseg > 1 else 0)
-        cands = [(0, 0, 0)]
-        pairs_ok = self.net.tc_tune_pairs and (d.B * d.H * d.W) >= 256 and d.N >= 128
-        for bn in (32, 64, 128, 160, 256):
-            if d.N % bn != 0 and d.N > bn:
-                continue
-            if d.N <= bn // 2 and bn > 32:
-                continue
-            for sp in (1, 2, 3, 4, 6, 8, 12, 16, 24):
-                if sp > 1 and total_kb // sp < 4:
-                    continue
-                cands.append((bn, sp, 0))
-                if pairs_ok and bn >= 128 and sp <= 8:
-                    cands.append((bn, sp, 2))               # cta_group::2 CTA pairs (halves the B-tile bytes each SM ingests)
-        best, best_t, auto_t = (0, 0, 0), float("inf"), None
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        REPS = 6
-
-        def timed(launch):
-            """REPS x (evict the weights from L2, pull the activations back in, launch) in one event-timed region: the event
-            clock ticks in ~2 us steps, far too coarse for one 15 us launch."""
-            e0.record()
-            for _ in range(REPS):
-                self._tune_flush.zero_()
-                a_tensor.view(torch.int16).max()
-                if launch is not None and launch() != 0:
-                    return None
-            e1.record()
-            e1.synchronize()
-            return e0.elapsed_time(e1) / REPS
-
-        timed(None)
-        base = min(timed(None), timed(None))                 # cost of the eviction + touch alone
-        for bn, sp, two in cands:
-            d.block_n, d.splits, d.two_cta = bn, sp, two
-            h = C.c_void_p()
-            if lib.sdk_tc_gemm_create(C.byref(d), C.byref(h)) != 0:
-                continue
-            ws = torch.zeros(max(int(lib.sdk_tc_gemm_workspace_bytes(h)), 256), dtype=torch.uint8, device=self.device)
-            ok = lib.sdk_tc_gemm_set_workspace(h, ws.data_ptr()) == 0
-            if ok and cs is not None:
-                ok = lib.sdk_tc_gemm_set_stats(h, cs.data_ptr()) in (0, -3)
-            tmin = None
-            if ok:
-                ts = [timed(lambda: lib.sdk_tc_gemm_launch(h, stream)) for _ in range(3)]
-                if None not in ts:
-                    tmin = min(ts) - base
-            torch.cuda.synchronize(self.device)
-            lib.sdk_tc_gemm_destroy(h)
-            if tmin is not None:
-                if (bn, sp, two) == (0, 0, 0):
-                    auto_t = tmin
-                if tmin < best_t:
-                    best, best_t = (bn, sp, two), tmin
-        # keep the model's choice unless a candidate is clearly (> 4 %) faster: timing noise must not flip tilings
-        if auto_t is not None and best_t > 0.96 * auto_t:
-            best = (0, 0, 0)
-        StepProgram._tune_cache[key] = best
-        StepProgram._tune_save(key, best)
-        if self.net.tc_autotune > 2:
-            print(f"autotune B{d.B} {d.H}x{d.W} C{d.C[0]} k{d.ksize[0]} N{d.N}: model {auto_t * 1e3 if auto_t else -1:.1f} us -> "
-                  f"{best} {best_t * 1e3:.1f} us", flush=True)
-        return best
-
-    def _gn(self, srcs, B, HW, g, b, eps, silu, want_raw=False):
-        """GroupNorm(32)(+SiLU) over the concat of srcs -> operand-typed tensor [B*HW, C]."""
-        Ct = sum(c for _, c in srcs)
-        s0, c0 = srcs[0]
-        s1, c1 = (srcs[1] if len(srcs) > 1 else (None, 0))
-        out = self.pool.get(B * HW, Ct, self.act)
-        raw = self.pool.get(B * HW, Ct, self.act) if want_raw else None
-        s1p = s1.data_ptr() if s1 is not None else 0
-        rawp = raw.data_ptr() if raw is not None else 0
-        mode = self.net.gn_mode
-        if self.gn_from_sums and all(getattr(sr, "_cstats", None) is not None for sr, _ in srcs):
-            cs0 = s0._cstats.data_ptr()
-            cs1 = s1._cstats.data_ptr() if s1 is not None else 0
-            self._emit(self.lib.sdk_groupnorm_apply_cs, s0.data_ptr(), c0, cs0, s1p, c1, cs1, B, HW, float(eps),
-                       g.data_ptr(), b.data_ptr(), int(silu), out.data_ptr(), rawp, self.act)
-            return out, raw
-        if mode == "sums":
-            mode = "split"
-        if mode == "auto":
-            # small tensors are latency-bound: one cluster launch (DSMEM reduce) beats two launches + ticketed tail;
-            # large ones are bandwidth-bound and need the whole chip (measured on B200, see DESIGN.md)
-            mode = "cluster" if B * HW * Ct * 4 <= self.net.gn_cluster_max_bytes else "split"
-        if mode == "cluster":
-            self._emit(self.lib.sdk_groupnorm_cluster, s0.data_ptr(), c0, s1p, c1, B, HW, float(eps), g.data_ptr(), b.data_ptr(),
-                       int(silu), out.data_ptr(), rawp, self.act)
-        elif mode == "coop":
-            # one cooperative launch (statistics, grid barrier, apply).  Measured on B200 inside the step graph:
-            # 6.36 ms/step vs 6.15 ms/step for the two-kernel form below, so it is not the default.
-            self._emit(self.lib.sdk_groupnorm_fused, s0.data_ptr(), c0, s1p, c1, B, HW, float(eps), g.data_ptr(), b.data_ptr(),
-                       int(silu), out.data_ptr(), rawp, self.act, self.gn_ws.data_ptr())
-        else:
-            self._emit(self.lib.sdk_groupnorm_stats, s0.data_ptr(), c0, s1p, c1, B, HW, float(eps),
-                       self.gn_stats.data_ptr(), self.gn_ws.data_ptr())
-            self._emit(self.lib.sdk_groupnorm_apply, s0.data_ptr(), c0, s1p, c1, B, HW, self.gn_stats.data_ptr(),
-                       g.data_ptr(), b.data_ptr(), int(silu), out.data_ptr(), rawp, self.act)
-        return out, raw
-
-    def _ln(self, x, g, b, rows, Cc, eps=1e-5, out_code=None):
-        code = self.act if out_code is None else out_code
-        out = self.pool.get(rows, Cc, code)
-        self._emit(self.lib.sdk_layernorm, x.data_ptr(), g.data_ptr(), b.data_ptr(), float(eps), out.data_ptr(), code, rows, Cc)
-        return out
-
-    def _linear_ln(self, a, w, bias, residual, g, b, rows, K, N, eps=1e-5):
-        """out = a W^T + bias + residual (fp32) and LayerNorm(out) (bf16) in one launch (sdk_linear_ln), or None when the shape is
-        not taken (row width not 160k / 128k with k <= 8, or a grid of more than one wave: the persistent GEMM + LayerNorm pair
-        overlaps epilogues across tiles there)."""
-        if self.act == F32_T or not getattr(self.net, "ln_fuse", False):
-            return None
-        bn = 160 if (N % 160 == 0 and N // 160 <= 8) else (128 if (N % 128 == 0 and N // 128 <= 8) else 0)
-        if os.environ.get("SDB200_LLN_PREFER128", "1") != "0" and N % 128 == 0 and N // 128 <= 8:
-            bn = 128                                           # the library's own preference (N = 640: clusters of 5)
-        max_ctas = self.net.ln_fuse_max_ctas
-        if max_ctas <= 0:
-            if not hasattr(self, "_sm_count"):
-                info = (C.c_int * 4)()
-                with torch.cuda.device(self.device):
-                    _lib.check(self.lib.sdk_device_info(info, 4))
-                self._sm_count = int(info[0])
-            max_ctas = self._sm_count
-        if not bn or K % 64 != 0 or ((rows + 127) // 128) * (N // bn) > max_ctas:
-            return None
-        out = self.pool.get(rows, N, F32_T)
-        ln = self.pool.get(rows, N, BF16_T)
-        d = LinearLnDesc()
-        d.a, d.w, d.bias = a.data_ptr(), w.data_ptr(), (bias.data_ptr() if bias is not None else 0)
-        d.residual = residual.data_ptr() if residual is not None else 0
-        d.out, d.ln_out, d.gamma, d.beta, d.eps = out.data_ptr(), ln.data_ptr(), g.data_ptr(), b.data_ptr(), float(eps)
-        d.M, d.K, d.N = rows, K, N
-        h = C.c_void_p()
-        rc = self.lib.sdk_linear_ln_create(C.byref(d), C.byref(h))
-        if rc == -3:
-            self.pool.put(out)
-            self.pool.put(ln)
-            return None
-        _lib.check(rc)
-        self.lln_handles.append(h)
-        self.keep.append(d)
-        self._handle_meta.append([3, h, d, 0])
-        self._emit(self.lib.sdk_linear_ln_launch, h)
-        return out, ln
-
-    def _attention(self, q, q_row, q_batch, k, k_row, k_batch, v, v_row, v_batch, B, heads, Sq, Sk, D, Cc, causal=False):
-        out = self.pool.get(B * Sq, Cc, self.act)
-        if self.act != F32_T and D in (40, 64, 80, 160) and self.net.attn_tc:
-            # tcgen05 flash attention (S and P.V on the tensor core, thread-per-row softmax)
-            h = C.c_void_p()
-            _lib.check(self.lib.sdk_attention_tc_create(q, q_row, q_batch, k, k_row, k_batch, v, v_row, v_batch,
-                                                        out.data_ptr(), Cc, Sq * Cc, B, heads, Sq, Sk, D, float(D ** -0.5), C.byref(h)))
-            if causal:
-                _lib.check(self.lib.sdk_attention_tc_set_causal(h, 1))
-            ad = AttentionTcDesc()
-            ad.q, ad.k, ad.v, ad.out = q, k, v, out.data_ptr()
-            ad.q_row, ad.q_batch, ad.k_row, ad.k_batch, ad.v_row, ad.v_batch = q_row, q_batch, k_row, k_batch, v_row, v_batch
-            ad.o_row, ad.o_batch, ad.B, ad.heads, ad.Sq, ad.Sk, ad.D, ad.scale = Cc, Sq * Cc, B, heads, Sq, Sk, D, float(D ** -0.5)
-            self.keep.append(ad)
-            self._handle_meta.append([2, h, ad, int(bool(causal))])
-            self.attn_handles.append(h)
-            self._emit(self.lib.sdk_attention_tc_launch, h)
-            return out
+        # time embedding (unet.py:209-220) + all 22 ResBlock time projections (unet.py:182-183)
+        te0 = torch.empty((self.nt, a.t_embed_dim), dtype=f32, device=dev)
+        te1 = torch.empty((self.nt, a.temb), dtype=f32, device=dev)
+        te2 = torch.empty((self.nt, a.temb), dtype=f32, device=dev)
+        self.tb = torch.empty((self.nt, a.tb_total), dtype=f32, device=dev)
+        self.keep += [te0, te1, te2]
+        t_first = len(self.ops)
+        self._emit(lib.sdk_time_sinusoid, self.t_in.data_ptr(), self.nt, a.t_embed_dim, te0.data_ptr())
+        self._emit(lib.sdk_gemv, t["time_embedding.ffn.0.weight"].data_ptr(), F32_T, t["time_embedding.ffn.0.bias"].data_ptr(),
+                   te0.data_ptr(), te1.data_ptr(), self.nt, a.temb, a.t_embed_dim, 0, 1)
+        self._emit(lib.sdk_gemv, t["time_embedding.ffn.2.weight"].data_ptr(), F32_T, t["time_embedding.ffn.2.bias"].data_ptr(),
+                   te1.data_ptr(), te2.data_ptr(), self.nt, a.temb, a.temb, 0, 0)
+        self._emit(lib.sdk_gemv, t["tb.w"].data_ptr(), self.pw.wcode, t["tb.b"].data_ptr(),
+                   te2.data_ptr(), self.tb.data_ptr(), self.nt, a.tb_total, a.temb, 1, 0)
+        self.time_ops = self.ops[t_first:]       # timestep -> self.tb; a sampling loop precomputes them for its whole grid
+        # context operand (context program)
         if self.act == F32_T:
-            self._emit(self.lib.sdk_attention_f32_ex, q, q_row, q_batch, k, k_row, k_batch, v, v_row, v_batch,
-                       out.data_ptr(), Cc, Sq * Cc, B, heads, Sq, Sk, D, float(D ** -0.5), int(causal))
-            return out
-        if causal:
-            raise RuntimeError("causal attention in bf16 needs the tcgen05 kernel (head_dim 40/64/80/160, SDB200_ATTN_TC=1)")
-        self._emit(self.lib.sdk_attention_bf16, q, q_row, q_batch, k, k_row, k_batch, v, v_row, v_batch,
-                   out.data_ptr(), Cc, Sq * Cc, B, heads, Sq, Sk, D, float(D ** -0.5))
-        return out
-
-    # ---- blocks -----------------------------------------------------------------------
-    def _res(self, r: ResBlock, srcs, B, H, W):
-        """models/unet/unet.py:174-195."""
-        t, HW = self.pw.t, H * W
-        p = r.prefix
-        need_raw = r.has_proj and self.act != F32_T
-        a1, raw = self._gn(srcs, B, HW, t[f"{p}.groupnorm_1.g"], t[f"{p}.groupnorm_1.b"], r.eps, True, want_raw=need_raw)
-        tb_ptr = self.tb.data_ptr() + 4 * r.tb_offset
-        h1, _, _ = self._conv([(a1, r.cin_total)], t[f"{p}.conv_1.w"], t[f"{p}.conv_1.b"], B, H, W, r.cout, k=3,
-                              tbias=tb_ptr, tb_stride=(self.arch.tb_total if self.nt > 1 else 0), want_stats=True)
-        self.pool.put(a1)
-        a2, _ = self._gn([(h1, r.cout)], B, HW, t[f"{p}.groupnorm_2.g"], t[f"{p}.groupnorm_2.b"], r.eps, True)
-        self.pool.put(h1)
-        if r.has_proj:
-            if self.act == F32_T:
-                sc, _, _ = self._conv(srcs, t[f"{p}.proj.w"], t[f"{p}.proj.b"], B, H, W, r.cout, k=1)
-                out, _, _ = self._conv([(a2, r.cout)], t[f"{p}.conv_2.w"], t[f"{p}.conv_2.b"], B, H, W, r.cout, k=3, residual=sc,
-                                       want_stats=True)
-                self.pool.put(sc)
-            else:
-                # 1x1 shortcut conv (unet.py:192) as a second K segment of conv_2's GEMM: same TMEM accumulator,
-                # no fp32 round trip of the shortcut tensor; bias = conv_2.bias + proj_input.bias (packed)
-                out, _, _ = self._conv([(a2, r.cout)], t[f"{p}.conv_2.w"], t[f"{p}.conv2_proj.b"], B, H, W, r.cout, k=3,
-                                       seg2=(raw, r.cin_total, t[f"{p}.proj.w"]), want_stats=True)
-                self.pool.put(raw)
+            self.cond_act = self.cond_in.view(self.Bc * self.Sk, a.dctx)
         else:
-            out, _, _ = self._conv([(a2, r.cout)], t[f"{p}.conv_2.w"], t[f"{p}.conv_2.b"], B, H, W, r.cout, k=3,
-                                   residual=srcs[0][0], want_stats=True)
-        self.pool.put(a2)
-        return out
+            self.cond_act = torch.empty((self.Bc * self.Sk, a.dctx), dtype=_DT[self.act], device=dev)
+            self._emit(lib.sdk_cast_upsample, self.cond_in.data_ptr(), self.cond_act.data_ptr(), self.act,
+                       1, 1, self.Bc * self.Sk, a.dctx, 1, ctx=True)
+
+        self.kv_all = None
+        if self.pw.kv_total:
+            self.kv_all = torch.empty((self.Bc * self.Sk, self.pw.kv_total), dtype=_DT[self.act], device=dev)
+            self._conv([(self.cond_act, a.dctx)], t["kv2_all.w"], None, 1, 1, self.Bc * self.Sk, self.pw.kv_total,
+                       out_code=self.act, out=self.kv_all, ctx=True)
+        # conv_in (unet.py:256): NCHW latent -> NHWC, then 3x3 conv with Cin = 4 (FFMA kernel: K = 36)
+        xin = self.pool.get(B * H * W, a.in_channels, F32_T)
+        self._emit(lib.sdk_nchw_to_nhwc, self.x_in.data_ptr(), xin.data_ptr(), self.b_src, B, a.in_channels, H * W)
+        x = self._conv_in(xin, a.in_channels, B, H, W, BLOCK_OUT[0])
+        self.pool.put(xin)
+        skips = [(x, BLOCK_OUT[0], H, W)]
+        h, w = H, W
+        xc = BLOCK_OUT[0]
+        shared = {id(x)}                      # tensors referenced by the skip stack must not be recycled early
+        tb_stride = a.tb_total if nt > 1 else 0
+
+        def res(r, srcs, h, w):               # models/unet/unet.py:174-195
+            return self._resblock(r.prefix, srcs, r.cout, r.eps, B, h, w, tbias=self.tb.data_ptr() + 4 * r.tb_offset,
+                                  tb_stride=tb_stride)
+
+        def release(tensor):
+            if id(tensor) not in shared:
+                self.pool.put(tensor)
+
+        for st in a.down:
+            for r, tr in st.blocks:
+                y = res(r, [(x, xc)], h, w)
+                release(x)
+                x, xc = y, r.cout
+                if tr is not None:
+                    y = self._transformer(tr, x, B, h, w)
+                    self.pool.put(x)
+                    x = y
+                skips.append((x, xc, h, w))
+                shared.add(id(x))
+            if st.resample is not None:
+                wn, bn_ = t[f"{st.resample.prefix}.w"], t[f"{st.resample.prefix}.b"]
+                if self.act == F32_T:
+                    y, h, w = self._conv([(x, xc)], wn, bn_, B, h, w, xc, k=3, stride=2, want_stats=True)
+                else:
+                    # stride-2 3x3 (unet.py:236): the A boxes walk the bf16 input with element stride 2 (no im2col matrix) ...
+                    ho, wo = (h - 1) // 2 + 1, (w - 1) // 2 + 1
+                    y = None
+                    if self.net.fold_gathers and B * ho * wo >= self.net.fold_min_rows_s2:
+                        op, _ = self._operand(x, B, h, w, xc)
+                        y, _, _ = self._conv([(op, xc)], wn, bn_, B, h, w, xc, k=3, stride=2, want_stats=True, fold_gather=True)
+                        self.pool.put(op)
+                    if y is None:
+                        # ... or, for shapes the fold does not take: gather the 9 taps into bf16 rows, then a 1-tap tensor-core GEMM
+                        col = self.pool.get(B * ho * wo, 9 * xc, BF16_T)
+                        self._emit(lib.sdk_im2col_s2, x.data_ptr(), col.data_ptr(), B, h, w, xc)
+                        y, _, _ = self._conv([(col, 9 * xc)], wn, bn_, B, ho, wo, xc, k=1, want_stats=True)
+                        self.pool.put(col)
+                    h, w = ho, wo
+                x = y
+                skips.append((x, xc, h, w))
+                shared.add(id(x))
+        # bottleneck (unet.py:383-391)
+        y = res(a.mid[0], [(x, xc)], h, w)
+        x = y                                   # previous x is still on the skip stack
+        y = self._transformer(a.mid[1], x, B, h, w)
+        self.pool.put(x)
+        x = y
+        y = res(a.mid[2], [(x, xc)], h, w)
+        self.pool.put(x)
+        x = y
+        # decoder (unet.py:337-351)
+        for st in a.up:
+            prev_w = skips[-1][3]
+            for r, tr in st.blocks:
+                sk, skc, sh, sw = skips.pop()
+                if (sh, sw) != (h, w):
+                    raise RuntimeError(f"Sizes of tensors must match except in dimension 1 (skip {sh}x{sw} vs x {h}x{w}); "
+                                       "latent H and W must be multiples of 8 (reference: unet.py:343)")
+                y = res(r, [(x, xc), (sk, skc)], h, w)
+                self.pool.put(x)
+                shared.discard(id(sk))
+                self.pool.put(sk)
+                x, xc = y, r.cout
+                if tr is not None:
+                    y = self._transformer(tr, x, B, h, w)
+                    self.pool.put(x)
+                    x = y
+            if st.resample is not None:
+                up = not (skips and skips[-1][3] == prev_w)          # unet.py:346-349
+                y, h, w = self._upsample_conv(st.resample.prefix, x, xc, B, h, w, up=up)
+                self.pool.put(x)
+                x = y
+        # head (unet.py:398-401): GN + SiLU + conv 320 -> out_channels, written straight to NCHW
+        ao, _ = self._gn([(x, xc)], B, h * w, t["out.gn.g"], t["out.gn.b"], a.eps, True)
+        self.pool.put(x)
+        self._conv([(ao, xc)], t["out.w"], t["out.b"], B, h, w, a.out_channels, k=3, out=self.out, out_nchw=True)
+        self.pool.put(ao)
+
+    def _finish(self):
+        super()._finish()
+        self.body_ops = [op for op in self.ops if all(op is not o for o in self.time_ops)]     # the step without the time embedding
+
+    def _scratch(self):
+        return super()._scratch() + [self.tb, self.cond_act, self.kv_all] + list(self.kv.values())
 
     def _transformer(self, tr: Transformer, x, B, H, W):
         """models/unet/unet.py:73-91 + 127-150 + attention.py:70-87, on [B*HW, C] tokens (NHWC == tokens)."""
@@ -808,319 +379,14 @@ class StepProgram:
         self.pool.put(h4)
         return out
 
-    def _operand(self, x, B, H, W, Cc, up=1):
-        """fp32 residual-stream tensor -> GEMM operand type (identity on the fp32 path)."""
-        if self.act == F32_T and up == 1:
-            return x, False
-        o = self.pool.get(B * H * up * W * up, Cc, self.act)
-        self._emit(self.lib.sdk_cast_upsample, x.data_ptr(), o.data_ptr(), self.act, B, H, W, Cc, up)
-        return o, True
-
-    # ---- whole network ------------------------------------------------------------------
-    def _build(self):
-        a, t, lib = self.arch, self.pw.t, self.lib
-        B, H, W = self.B, self.H, self.W
-        dev, f32 = self.device, torch.float32
-        # time embedding (unet.py:209-220) + all 22 ResBlock time projections (unet.py:182-183)
-        te0 = torch.empty((self.nt, a.t_embed_dim), dtype=f32, device=dev)
-        te1 = torch.empty((self.nt, a.temb), dtype=f32, device=dev)
-        te2 = torch.empty((self.nt, a.temb), dtype=f32, device=dev)
-        self.tb = torch.empty((self.nt, a.tb_total), dtype=f32, device=dev)
-        self.keep += [te0, te1, te2]
-        t_first = len(self.ops)
-        self._emit(lib.sdk_time_sinusoid, self.t_in.data_ptr(), self.nt, a.t_embed_dim, te0.data_ptr())
-        self._emit(lib.sdk_gemv, t["time_embedding.ffn.0.weight"].data_ptr(), F32_T, t["time_embedding.ffn.0.bias"].data_ptr(),
-                   te0.data_ptr(), te1.data_ptr(), self.nt, a.temb, a.t_embed_dim, 0, 1)
-        self._emit(lib.sdk_gemv, t["time_embedding.ffn.2.weight"].data_ptr(), F32_T, t["time_embedding.ffn.2.bias"].data_ptr(),
-                   te1.data_ptr(), te2.data_ptr(), self.nt, a.temb, a.temb, 0, 0)
-        self._emit(lib.sdk_gemv, t["tb.w"].data_ptr(), self.pw.wcode, t["tb.b"].data_ptr(),
-                   te2.data_ptr(), self.tb.data_ptr(), self.nt, a.tb_total, a.temb, 1, 0)
-        self.time_ops = self.ops[t_first:]       # timestep -> self.tb; a sampling loop precomputes them for its whole grid
-        self._time_range = (t_first, len(self.ops))
-        # context operand (context program)
-        if self.act == F32_T:
-            self.cond_act = self.cond_in.view(self.Bc * self.Sk, a.dctx)
-        else:
-            self.cond_act = torch.empty((self.Bc * self.Sk, a.dctx), dtype=_DT[self.act], device=dev)
-            self._emit(lib.sdk_cast_upsample, self.cond_in.data_ptr(), self.cond_act.data_ptr(), self.act,
-                       1, 1, self.Bc * self.Sk, a.dctx, 1, ctx=True)
-
-        self.kv_all = None
-        if self.pw.kv_total:
-            self.kv_all = torch.empty((self.Bc * self.Sk, self.pw.kv_total), dtype=_DT[self.act], device=dev)
-            self._conv([(self.cond_act, a.dctx)], t["kv2_all.w"], None, 1, 1, self.Bc * self.Sk, self.pw.kv_total,
-                       out_code=self.act, out=self.kv_all, ctx=True)
-        # conv_in (unet.py:256): NCHW latent -> NHWC, then 3x3 conv with Cin = 4 (FFMA kernel: K = 36)
-        xin = self.pool.get(B * H * W, a.in_channels, F32_T)
-        self._emit(lib.sdk_nchw_to_nhwc, self.x_in.data_ptr(), xin.data_ptr(), self.b_src, B, a.in_channels, H * W)
-        if a.in_channels == 4:
-            # dedicated K = 36 kernel; also accumulates the statistics table of the first GroupNorm
-            x = self.pool.get(B * H * W, BLOCK_OUT[0], F32_T)
-            cs = self._stat_table(B, BLOCK_OUT[0]) if self.gn_from_sums else None
-            w_t = t["conv_in.w"].float().reshape(BLOCK_OUT[0], 36).t().contiguous()        # [kh][kw][cin][N]
-            self.keep.append(w_t)
-            self.consts.append(w_t)
-            self._emit(lib.sdk_conv_in, xin.data_ptr(), w_t.data_ptr(), t["conv_in.b"].data_ptr(), x.data_ptr(),
-                       cs.data_ptr() if cs is not None else 0, B, H, W, BLOCK_OUT[0])
-            if cs is not None:
-                x._cstats = cs
-        else:
-            x, _, _ = self._conv([(xin, a.in_channels)], t["conv_in.w"], t["conv_in.b"], B, H, W, BLOCK_OUT[0], k=3,
-                                 in_code=F32_T, force_simt=True, want_stats=True)
-        self.pool.put(xin)
-        skips = [(x, BLOCK_OUT[0], H, W)]
-        h, w = H, W
-        xc = BLOCK_OUT[0]
-        shared = {id(x)}                      # tensors referenced by the skip stack must not be recycled early
-
-        def release(tensor):
-            if id(tensor) not in shared:
-                self.pool.put(tensor)
-
-        for st in a.down:
-            for r, tr in st.blocks:
-                y = self._res(r, [(x, xc)], B, h, w)
-                release(x)
-                x, xc = y, r.cout
-                if tr is not None:
-                    y = self._transformer(tr, x, B, h, w)
-                    self.pool.put(x)
-                    x = y
-                skips.append((x, xc, h, w))
-                shared.add(id(x))
-            if st.resample is not None:
-                wn, bn_ = t[f"{st.resample.prefix}.w"], t[f"{st.resample.prefix}.b"]
-                if self.act == F32_T:
-                    y, h, w = self._conv([(x, xc)], wn, bn_, B, h, w, xc, k=3, stride=2, want_stats=True)
-                else:
-                    # stride-2 3x3 (unet.py:236): the A boxes walk the bf16 input with element stride 2 (no im2col matrix) ...
-                    ho, wo = (h - 1) // 2 + 1, (w - 1) // 2 + 1
-                    y = None
-                    if self.net.fold_gathers and B * ho * wo >= self.net.fold_min_rows_s2:
-                        op, _ = self._operand(x, B, h, w, xc)
-                        y, _, _ = self._conv([(op, xc)], wn, bn_, B, h, w, xc, k=3, stride=2, want_stats=True, fold_gather=True)
-                        self.pool.put(op)
-                    if y is None:
-                        # ... or, for shapes the fold does not take: gather the 9 taps into bf16 rows, then a 1-tap tensor-core GEMM
-                        col = self.pool.get(B * ho * wo, 9 * xc, BF16_T)
-                        self._emit(lib.sdk_im2col_s2, x.data_ptr(), col.data_ptr(), B, h, w, xc)
-                        y, _, _ = self._conv([(col, 9 * xc)], wn, bn_, B, ho, wo, xc, k=1, want_stats=True)
-                        self.pool.put(col)
-                    h, w = ho, wo
-                x = y
-                skips.append((x, xc, h, w))
-                shared.add(id(x))
-        # bottleneck (unet.py:383-391)
-        y = self._res(a.mid[0], [(x, xc)], B, h, w)
-        x = y                                   # previous x is still on the skip stack
-        y = self._transformer(a.mid[1], x, B, h, w)
-        self.pool.put(x)
-        x = y
-        y = self._res(a.mid[2], [(x, xc)], B, h, w)
-        self.pool.put(x)
-        x = y
-        # decoder (unet.py:337-351)
-        for st in a.up:
-            prev_w = skips[-1][3]
-            for r, tr in st.blocks:
-                sk, skc, sh, sw = skips.pop()
-                if (sh, sw) != (h, w):
-                    raise RuntimeError(f"Sizes of tensors must match except in dimension 1 (skip {sh}x{sw} vs x {h}x{w}); "
-                                       "latent H and W must be multiples of 8 (reference: unet.py:343)")
-                y = self._res(r, [(x, xc), (sk, skc)], B, h, w)
-                self.pool.put(x)
-                shared.discard(id(sk))
-                self.pool.put(sk)
-                x, xc = y, r.cout
-                if tr is not None:
-                    y = self._transformer(tr, x, B, h, w)
-                    self.pool.put(x)
-                    x = y
-            if st.resample is not None:
-                up = not (skips and skips[-1][3] == prev_w)          # unet.py:346-349
-                rp = st.resample.prefix
-                y = None
-                if up and self.act != F32_T and self.net.fold_gathers and B * h * w >= self.net.fold_min_rows_up:
-                    # nearest-2x upsample folded into the conv: four 2x2 convs on the low-res bf16 input, one per output parity
-                    op, tmp = self._operand(x, B, h, w, xc)
-                    y, hn, wn_ = self._conv([(op, xc)], t[f"{rp}.w_up2"], t[f"{rp}.b"], B, h, w, xc, k=3, up=True, want_stats=True, fold_gather=True)
-                    if y is None:
-                        self.pool.put(op)
-                        tmp = False
-                    else:
-                        h, w = hn, wn_
-                if y is None:
-                    op, tmp = self._operand(x, B, h, w, xc, up=2 if (up and self.act != F32_T) else 1)
-                    if up and self.act != F32_T:
-                        y, h, w = self._conv([(op, xc)], t[f"{rp}.w"], t[f"{rp}.b"], B, 2 * h, 2 * w, xc, k=3, want_stats=True)
-                    else:
-                        y, h, w = self._conv([(op, xc)], t[f"{rp}.w"], t[f"{rp}.b"], B, h, w, xc, k=3, up=up, want_stats=True)
-                if tmp:
-                    self.pool.put(op)
-                self.pool.put(x)
-                x = y
-        # head (unet.py:398-401): GN + SiLU + conv 320 -> out_channels, written straight to NCHW
-        ao, _ = self._gn([(x, xc)], B, h * w, t["out.gn.g"], t["out.gn.b"], a.eps, True)
-        self.pool.put(x)
-        self._conv([(ao, xc)], t["out.w"], t["out.b"], B, h, w, a.out_channels, k=3, out=self.out, out_nchw=True)
-        self.pool.put(ao)
-        self.n_launch = len(self.ops)
-        self._finish_tc()
-
-    def _finish_tc(self):
-        """One zeroed split-K workspace shared by every tensor-core GEMM of the program (stream-ordered)."""
-        need = max([int(self.lib.sdk_tc_gemm_workspace_bytes(h)) for h in self.tc_handles] + [0])
-        self.tc_ws = torch.zeros(max(need, 256), dtype=torch.uint8, device=self.device)
-        for h in self.tc_handles:
-            _lib.check(self.lib.sdk_tc_gemm_set_workspace(h, self.tc_ws.data_ptr()))
-        t0, t1 = self._time_range
-        self.body_ops = self.ops[:t0] + self.ops[t1:]       # the step without the time-embedding chain
-        if self.gn_from_sums:                               # first op of the step: zero every statistics table at once
-            zero = (self.lib.sdk_zero, (self.stat_arena.data_ptr(), self.stat_used))
-            self.ops.insert(0, zero)
-            self.body_ops.insert(0, zero)
-            self.n_launch = len(self.ops)
-
-    def tc_info(self):
-        out = []
-        buf = (C.c_int * 8)()
-        for h in self.tc_handles:
-            _lib.check(self.lib.sdk_tc_gemm_info(h, buf, 8))
-            out.append(tuple(buf))
-        return out
-
-    def __del__(self):
-        try:
-            if getattr(self, "plan", None) is not None:           # the plan owns the adopted handles
-                self.lib.sdk_plan_destroy(self.plan)
-                return
-            for h in getattr(self, "tc_handles", []):
-                self.lib.sdk_tc_gemm_destroy(h)
-            for h in getattr(self, "attn_handles", []):
-                self.lib.sdk_attention_tc_destroy(h)
-            for h in getattr(self, "lln_handles", []):
-                self.lib.sdk_linear_ln_destroy(h)
-        except Exception:
-            pass
-
-    # ---- plan-level C entry (include/sdb200.h: sdk_plan_*) -------------------------------------------------
-    # The launch lists live in an sdk_plan: one C call replays a program, sdk_plan_save writes an engine file that a host
-    # without Python / PyTorch loads and runs (tools/c_host/denoise.c).  Program ids of the package:
-    PROGRAM_IDS = {"ops": 0, "ctx_ops": 1, "time_ops": 2, "body_ops": 3}
-    PROGRAM_LOOP_STEP = 4
-
-    @staticmethod
-    def _slots(fn_name, args):
-        """Arguments of one recorded launch as the 64-bit slots sdk_plan_add_launch takes (floats as IEEE-754 bits)."""
-        types = _lib.SIGNATURES[fn_name][:-1]                # without the trailing stream
-        if len(types) != len(args):
-            raise RuntimeError(f"{fn_name}: {len(args)} recorded arguments, the binding table has {len(types)}")
-        out = (C.c_uint64 * max(len(args), 1))()
-        for i, (a, ty) in enumerate(zip(args, types)):
-            if ty is _lib.F32:
-                v = struct.unpack("<I", struct.pack("<f", float(a)))[0]
-            elif hasattr(a, "_obj"):                         # ctypes.byref(struct): the struct's host address (the plan copies it)
-                v = C.addressof(a._obj)
-            elif isinstance(a, C.c_void_p):
-                v = a.value or 0
-            elif a is None:
-                v = 0
-            else:
-                v = int(a) & 0xFFFFFFFFFFFFFFFF
-            out[i] = v
-        return out
-
-    def _ensure_plan(self):
-        if self.plan is not None:
-            return self.plan
-        lib = self.lib
-        h = C.c_void_p()
-        _lib.check(lib.sdk_plan_create(C.byref(h)))
-        ws = self.tc_ws.data_ptr() if getattr(self, "tc_ws", None) is not None else 0
-        for kind, hd, desc, aux in self._handle_meta:
-            a = (C.c_uint64 * 2)(aux, ws if kind == 1 else 0)
-            _lib.check(lib.sdk_plan_adopt(h, kind, hd, C.byref(desc), C.sizeof(desc), a, 2))
-        self.plan = h
-        return h
-
-    def plan_add(self, program, fn_name, args):
-        """Append one launch (entry-point name + arguments without the stream) to ``program`` of this plan."""
-        sl = self._slots(fn_name, args)
-        _lib.check(self.lib.sdk_plan_add_launch(self._ensure_plan(), program, fn_name.encode(), sl, len(args)))
-
-    def _program_of(self, ops):
-        """Program id of one of this object's launch lists (transcribed into the plan on first use), None for ad-hoc lists."""
-        pid = self._plan_ids.get(id(ops))
-        if pid is not None:
-            return pid
-        for name, pid in self.PROGRAM_IDS.items():
-            if getattr(self, name, None) is ops:
-                for fn, args in ops:
-                    self.plan_add(pid, fn.__name__, args)
-                self._plan_ids[id(ops)] = pid
-                return pid
-        return None
-
-    def plan_regions(self):
-        """(tensor, kind, name) of every device buffer the programs touch: kind 0 constant, 1 scratch, 2 named I/O."""
-        reg = [(t, 0, "") for t in self.pw.t.values()] + [(t, 0, "") for t in self.consts]
-        reg += [(raw, 1, "") for raw in self.pool.all]
-        for name in ("stat_arena", "gn_ws", "gn_stats", "tc_ws", "tb", "cond_act", "kv_all"):
-            t = getattr(self, name, None)
-            if t is not None:
-                reg.append((t, 1, ""))
-        reg += [(t, 1, "") for t in getattr(self, "kv", {}).values()]
-        reg += [(t, 1, "") for t in self.keep if isinstance(t, torch.Tensor) and all(t is not c for c in self.consts)]
-        for name, attr in (("x", "x_in"), ("timestep", "t_in"), ("context", "cond_in"), ("out", "out"),
-                           ("z", "z_in"), ("ids", "ids_in")):         # VAE decode: "z" -> "out"; text encoder: "ids" -> "out"
-            t = getattr(self, attr, None)
-            if t is not None:
-                reg.append((t, 2, name))
-        return reg
-
-    def export_engine(self, path, extra_regions=()):
-        """Write the engine file of this program set (sdk_plan_save): launch lists, descriptors with their tuned tilings, packed
-        weights.  A host without Python loads it with sdk_plan_load and runs program 1 (context) then 0 (forward)."""
-        plan = self._ensure_plan()
-        for name in self.PROGRAM_IDS:
-            ops = getattr(self, name, None)
-            if ops:
-                self._program_of(ops)
-        seen = set()
-        for t, kind, name in list(self.plan_regions()) + list(extra_regions):
-            nbytes = t.numel() * t.element_size()
-            key = (t.data_ptr(), nbytes)
-            if nbytes == 0 or key in seen:
-                continue
-            if kind != 2 and any(k[0] == key[0] for k in seen):           # a view of a buffer that is already registered
-                continue
-            seen.add(key)
-            _lib.check(self.lib.sdk_plan_add_region(plan, t.data_ptr(), nbytes, kind, name.encode()))
-        torch.cuda.synchronize(self.device)
-        with torch.cuda.device(self.device):
-            _lib.check(self.lib.sdk_plan_save(plan, os.fsencode(path)))
-
-    # ---- execution ----------------------------------------------------------------------
-    def launch(self, ops):
-        with torch.cuda.device(self.device):                    # the library keys its per-device state on the CURRENT device
-            stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-            pid = self._program_of(ops)
-            if pid is not None:                                 # the program's launch list lives in the C plan: one call
-                rc = self.lib.sdk_plan_launch(self.plan, pid, stream)
-                if rc != 0:
-                    _lib.check(rc)
-                return
-            for fn, args in ops:
-                rc = fn(*args, stream)
-                if rc != 0:
-                    _lib.check(rc)
-
 
 # ======================================================================================
 # module
 # ======================================================================================
-class UNet(nn.Module):
+class UNet(ProgramModule):
     """Drop-in for the reference ``UNet`` (models/unet/unet.py:353-461)."""
+
+    NORM_PARAMS = ("output.0",)             # the head's GroupNorm (unet.py:398) is the first module of a Sequential
 
     def __init__(self,
                  attention_head_dim: Union[int, List[int]] = 8,
@@ -1142,57 +408,7 @@ class UNet(nn.Module):
             raise ValueError("in_channels > 8 is not supported by the conv_in kernel")
         self.arch = build_arch(attention_head_dim, cross_attention_dim, in_channels, out_channels, block_out_channels,
                                down_block_types, t_embed_dim, num_attention_heads, eps)
-        for name, shape in param_spec(self.arch):
-            self._register(name, shape)
-        read_knobs(self)
-        self._packed: Dict = {}
-        self._plans: Dict = {}
-        self.register_load_state_dict_post_hook(lambda module, incompatible: module.invalidate())
-
-    # ---- parameters -------------------------------------------------------------------
-    def _register(self, name: str, shape):
-        parts = name.split(".")
-        node = self
-        for p in parts[:-1]:
-            if p not in node._modules:
-                node.add_module(p, _Node())
-            node = node._modules[p]
-        leaf, owner = parts[-1], parts[-2]
-        t = torch.empty(shape)
-        if "norm" in owner or name.startswith("output.0"):
-            t.fill_(1.0 if leaf == "weight" else 0.0)               # nn.GroupNorm / nn.LayerNorm defaults
-        else:
-            fan_in = 1
-            wshape = shape if leaf == "weight" else None
-            if wshape is None:                                      # bias: bound from the sibling weight's fan-in
-                wshape = tuple(getattr(node, "weight").shape)
-            for d in wshape[1:]:
-                fan_in *= d
-            bound = 1.0 / math.sqrt(fan_in)                         # nn.Conv2d / nn.Linear default init
-            t.uniform_(-bound, bound)
-        node.register_parameter(leaf, nn.Parameter(t, requires_grad=False))
-
-    def invalidate(self):
-        """Drop packed weights, plans and graphs (call after mutating parameters in place)."""
-        self._packed.clear()
-        self._plans.clear()
-
-    def _apply(self, fn, recurse=True):
-        # .to()/.cuda()/.float(): drop the packed copies only if the parameters really moved or changed type
-        # (the reference pipeline calls unet.to(device) before every generation, diffusion.py:222)
-        probe = next(self.parameters())
-        before = (probe.device, probe.dtype, probe.data_ptr())
-        out = super()._apply(fn, recurse)
-        probe = next(self.parameters())
-        if (probe.device, probe.dtype, probe.data_ptr()) != before:
-            self.invalidate()
-        return out
-
-    def set_precision(self, precision: str):
-        if precision not in ("fp32", "bf16"):
-            raise ValueError("precision must be 'fp32' or 'bf16'")
-        self.precision = precision
-        return self
+        self._init_params(param_spec(self.arch))
 
     # reference API no-ops (unet.py:404-428): inference path has no checkpointing; attention is always fused
     def gradient_checkpointing_enabled(self, enabled=False):
@@ -1272,14 +488,11 @@ class UNet(nn.Module):
         return model
 
 
-class _Runner:
-    """Executes a StepProgram: eager on the first call (also the warm-up), CUDA-graph replay afterwards."""
+class _Runner(GraphRunner):
+    """Runs a StepProgram; the context program runs only when ``cond`` is a new tensor or was written since the last call."""
 
     def __init__(self, prog: StepProgram, use_graph: bool):
-        self.prog = prog
-        self.use_graph = use_graph
-        self.graph = None
-        self.calls = 0
+        super().__init__(prog, use_graph)
         self._cond_ref = None
         self._cond_version = -1
 
@@ -1291,19 +504,5 @@ class _Runner:
             p.cond_in.copy_(cond, non_blocking=True)
             p.launch(p.ctx_ops)                       # cross-attention K/V: once per context, not per step
             self._cond_ref, self._cond_version = cond, tensor_version(cond)
-        self.calls += 1
-        with torch.cuda.device(p.device):
-            if not self.use_graph:
-                p.launch(p.ops)
-            elif self.graph is None:
-                if self.calls == 1:
-                    p.launch(p.ops)                       # eager warm-up (loads modules, sets func attributes)
-                else:
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        p.launch(p.ops)
-                    self.graph = g
-                    g.replay()
-            else:
-                self.graph.replay()
+        self.run()
         return p.out.clone()

@@ -17,60 +17,29 @@ import ctypes as C
 import json
 import math
 import os
-from typing import Dict
 
 import torch
-from torch import nn
 
-from . import _lib
-from ._lib import BF16_T, F32_T, ConvParams
+from ._lib import F32_T, ConvParams
 from .arch import vae_decoder_blocks, vae_param_spec
-from .unet import _DT, StepProgram, _Node, read_knobs
+from .program import GraphRunner, KernelWeights, LaunchProgram, ProgramModule
 
 SCALE = 0.18215                                            # models/vae/vae.py:271
 
 
-class VAEWeights:
+class VAEWeights(KernelWeights):
     """Kernel-layout copies of the decoder's parameters on one device for one precision."""
 
-    def __init__(self, net: "VAE", device, precision: str):
-        with torch.inference_mode(False), torch.no_grad():
-            self._pack(net, device, precision)
-
-    def _pack(self, net, device, precision):
-        self.device, self.precision = device, precision
-        wdt = torch.float32 if precision == "fp32" else torch.bfloat16
-        kmajor = precision != "fp32"
-        sd = {k: v.detach() for k, v in net.named_parameters()}
-        t: Dict[str, torch.Tensor] = {}
-
-        def dev(x, dt=torch.float32):
-            x = x.to(device=device, dtype=dt)
-            if kmajor and dt == torch.bfloat16 and x.dim() == 2 and x.shape[1] % 64 == 0:
-                n, k = x.shape                             # tensor-core operand: k-block-major [K/64][N][64]
-                x = x.view(n, k // 64, 64).permute(1, 0, 2)
-            return x.contiguous()
-
-        def conv_w(name, dt=wdt):
-            w = sd[name]
-            return dev(w.permute(0, 2, 3, 1).reshape(w.shape[0], -1), dt)
-
-        def res(p):
-            for n in ("norm1", "norm2"):
-                t[f"{p}.{n}.g"], t[f"{p}.{n}.b"] = dev(sd[f"{p}.{n}.weight"]), dev(sd[f"{p}.{n}.bias"])
-            for n in ("conv1", "conv2"):
-                t[f"{p}.{n}.w"], t[f"{p}.{n}.b"] = conv_w(f"{p}.{n}.weight"), dev(sd[f"{p}.{n}.bias"])
-            if f"{p}.conv_shortcut.weight" in sd:
-                t[f"{p}.sc.w"], t[f"{p}.sc.b"] = conv_w(f"{p}.conv_shortcut.weight"), dev(sd[f"{p}.conv_shortcut.bias"])
-                t[f"{p}.conv2_sc.b"] = dev(sd[f"{p}.conv2.bias"].float() + sd[f"{p}.conv_shortcut.bias"].float())
-
+    def _pack(self, net: "VAE"):
+        sd, t, dev, wdt = self.sd, self.t, self.dev, self.wdt
         # post_quant_conv (1x1, 4 -> 4) and conv_in (3x3, 4 -> 512): fp32 FFMA kernels in both modes (K = 4 / 36)
         t["pq.w"] = dev(sd["post_quant_conv.weight"].reshape(sd["post_quant_conv.weight"].shape[0], -1))
         t["pq.b"] = dev(sd["post_quant_conv.bias"])
-        w = sd["decoder.conv_in.weight"]
-        t["conv_in.w_t"] = dev(w.permute(0, 2, 3, 1).reshape(w.shape[0], -1).t())               # [kh][kw][cin][N]
-        t["conv_in.w"] = conv_w("decoder.conv_in.weight", torch.float32)
-        t["conv_in.b"] = dev(sd["decoder.conv_in.bias"])
+        self.conv_in("decoder.conv_in")
+
+        def res(p):
+            self.res_block(p, ("norm1", "norm2"), ("conv1", "conv2"), "conv_shortcut")
+
         res("decoder.mid_block.resnets.0")
         res("decoder.mid_block.resnets.1")
         a = "decoder.mid_block.attentions.0"
@@ -79,77 +48,32 @@ class VAEWeights:
             t[f"attn.{n}.w"], t[f"attn.{n}.b"] = dev(sd[f"{a}.{n}.weight"], wdt), dev(sd[f"{a}.{n}.bias"])
         # V is produced TRANSPOSED ([C][S] = W_v x^T: W_v is the A operand, the normalised tokens the B operand); its bias moves to
         # the P V GEMM because the softmax rows sum to one:  P (V + 1 b^T) = P V + b^T
-        t["attn.value.a"] = sd[f"{a}.value.weight"].to(device=device, dtype=wdt).contiguous()    # [C][C] row-major "activation"
+        t["attn.value.a"] = sd[f"{a}.value.weight"].to(device=self.device, dtype=wdt).contiguous()    # [C][C] row-major "activation"
         t["attn.value.b"] = dev(sd[f"{a}.value.bias"])
         for j, cin, cout, up in vae_decoder_blocks():
             for k in range(3):
                 res(f"decoder.up_blocks.{j}.resnets.{k}")
             if up:
-                p = f"decoder.up_blocks.{j}.upsamplers.0.conv"
-                t[f"{p}.w"], t[f"{p}.b"] = conv_w(f"{p}.weight"), dev(sd[f"{p}.bias"])
-                if precision != "fp32":                   # four parity sets of 2x2 taps (see unet.PackedWeights)
-                    w = sd[f"{p}.weight"].to(device=device, dtype=torch.float32).permute(0, 2, 3, 1)
-                    rows = {0: ([0], [1, 2]), 1: ([0, 1], [2])}
-                    sets = []
-                    for py in (0, 1):
-                        for px in (0, 1):
-                            wp = torch.zeros((w.shape[0], 2, 2, w.shape[3]), dtype=torch.float32, device=device)
-                            for ia in (0, 1):
-                                for ib in (0, 1):
-                                    for kh in rows[py][ia]:
-                                        for kw in rows[px][ib]:
-                                            wp[:, ia, ib] += w[:, kh, kw]
-                            sets.append(dev(wp.reshape(w.shape[0], -1), torch.bfloat16))
-                    t[f"{p}.w_up2"] = torch.cat(sets, 0).contiguous()
+                self.upsample_conv(f"decoder.up_blocks.{j}.upsamplers.0.conv")
         t["out.gn.g"], t["out.gn.b"] = dev(sd["decoder.conv_norm_out.weight"]), dev(sd["decoder.conv_norm_out.bias"])
-        t["out.w"], t["out.b"] = conv_w("decoder.conv_out.weight", wdt), dev(sd["decoder.conv_out.bias"])
-        self.t = t
+        t["out.w"], t["out.b"] = self.conv_w("decoder.conv_out.weight", wdt), dev(sd["decoder.conv_out.bias"])
 
 
-class VAEDecodeProgram(StepProgram):
+class VAEDecodeProgram(LaunchProgram):
     """``VAE.decode`` for a fixed (B, h, w) latent shape as a flat launch list (models/vae/vae.py:229-241,270-274)."""
+
+    IO_REGIONS = (("out", "out"), ("z", "z_in"))
 
     def __init__(self, net: "VAE", pw: VAEWeights, B, h, w):
         if h % 8 or w % 8:
             raise RuntimeError(f"latent {h}x{w}: height and width must be multiples of 8 (token count of the mid-block attention)")
-        with torch.inference_mode(False), torch.no_grad(), torch.cuda.device(pw.device):
-            self._init_common(net, pw, B)
-            self.h, self.w = h, w
-            # statistics kernels of the fp32 mode (bf16 takes them from the GEMM epilogues): sized for the final 8h x 8w image
-            self.gn_ws = torch.zeros(int(self.lib.sdk_groupnorm_workspace_bytes(B, 64 * h * w)), dtype=torch.uint8, device=pw.device)
-            self.gn_stats = torch.empty((B, 32, 2), dtype=torch.float32, device=pw.device)
-            self._build_decoder()
-
-    # ---- blocks -------------------------------------------------------------------------
-    def _vres(self, p, x, cin, cout, B, H, W):
-        """ResidualBlock (resnet.py:27-41): GN+SiLU -> conv3x3 -> GN+SiLU -> conv3x3 (+ 1x1 shortcut as a second K segment)."""
-        t, HW = self.pw.t, H * W
-        has_sc = cin != cout
-        need_raw = has_sc and self.act != F32_T
-        a1, raw = self._gn([(x, cin)], B, HW, t[f"{p}.norm1.g"], t[f"{p}.norm1.b"], 1e-6, True, want_raw=need_raw)
-        h1, _, _ = self._conv([(a1, cin)], t[f"{p}.conv1.w"], t[f"{p}.conv1.b"], B, H, W, cout, k=3, want_stats=True)
-        self.pool.put(a1)
-        a2, _ = self._gn([(h1, cout)], B, HW, t[f"{p}.norm2.g"], t[f"{p}.norm2.b"], 1e-6, True)
-        self.pool.put(h1)
-        if not has_sc:
-            out, _, _ = self._conv([(a2, cout)], t[f"{p}.conv2.w"], t[f"{p}.conv2.b"], B, H, W, cout, k=3, residual=x, want_stats=True)
-        elif self.act == F32_T:
-            sc, _, _ = self._conv([(x, cin)], t[f"{p}.sc.w"], t[f"{p}.sc.b"], B, H, W, cout, k=1)
-            out, _, _ = self._conv([(a2, cout)], t[f"{p}.conv2.w"], t[f"{p}.conv2.b"], B, H, W, cout, k=3, residual=sc, want_stats=True)
-            self.pool.put(sc)
-        else:
-            out, _, _ = self._conv([(a2, cout)], t[f"{p}.conv2.w"], t[f"{p}.conv2_sc.b"], B, H, W, cout, k=3,
-                                   seg2=(raw, cin, t[f"{p}.sc.w"]), want_stats=True)
-            self.pool.put(raw)
-        self.pool.put(a2)
-        return out
+        super().__init__(net, pw, B, h, w)
 
     def _vattention(self, x, Cc, B, H, W):
         """AttentionBlock (vae.py:121-134): GN -> q, k, v (with bias) -> softmax(q k^T / sqrt(C)) v -> proj -> + x, ONE head of
         dimension C.  Scores and P V are GEMMs whose B operand is an activation (row-major [N][K]); V is produced transposed."""
         t, S = self.pw.t, H * W
         M = B * S
-        dt = _DT[self.act]
         a, _ = self._gn([(x, Cc)], B, S, t["attn.gn.g"], t["attn.gn.b"], 1e-6, False)
         q, _, _ = self._conv([(a, Cc)], t["attn.query.w"], t["attn.query.b"], 1, 1, M, Cc, out_code=self.act)
         k, _, _ = self._conv([(a, Cc)], t["attn.key.w"], t["attn.key.b"], 1, 1, M, Cc, out_code=self.act)
@@ -172,10 +96,14 @@ class VAEDecodeProgram(StepProgram):
         return out
 
     # ---- whole decoder --------------------------------------------------------------------
-    def _build_decoder(self):
+    def _build(self, h, w):
         t, lib = self.pw.t, self.lib
-        B, h, w = self.B, self.h, self.w
+        B = self.B
         dev, f32 = self.device, torch.float32
+        self.h, self.w = h, w
+        # statistics kernels of the fp32 mode (bf16 takes them from the GEMM epilogues): sized for the final 8h x 8w image
+        self.gn_ws = torch.zeros(int(lib.sdk_groupnorm_workspace_bytes(B, 64 * h * w)), dtype=torch.uint8, device=dev)
+        self.gn_stats = torch.empty((B, 32, 2), dtype=f32, device=dev)
         zc = t["pq.w"].shape[0]
         top = t["conv_in.b"].shape[0]
         self.z_in = torch.empty((B, zc, h, w), dtype=f32, device=dev)
@@ -196,46 +124,24 @@ class VAEDecodeProgram(StepProgram):
         self._emit(lib.sdk_conv_gemm_f32, C.byref(p))
         self.pool.put(zn)
         # conv_in 3x3, 4 -> 512 (vae.py:231): the K = 36 kernel, which also reduces the first GroupNorm's statistics
-        if zc == 4:
-            x = self.pool.get(B * h * w, top, F32_T)
-            cs = self._stat_table(B, top) if self.gn_from_sums else None
-            self._emit(lib.sdk_conv_in, zq.data_ptr(), t["conv_in.w_t"].data_ptr(), t["conv_in.b"].data_ptr(), x.data_ptr(),
-                       cs.data_ptr() if cs is not None else 0, B, h, w, top)
-            if cs is not None:
-                x._cstats = cs
-        else:
-            x, _, _ = self._conv([(zq, zc)], t["conv_in.w"], t["conv_in.b"], B, h, w, top, k=3, in_code=F32_T, force_simt=True, want_stats=True)
+        x = self._conv_in(zq, zc, B, h, w, top)
         self.pool.put(zq)
         # mid block (vae.py:233-235)
-        y = self._vres("decoder.mid_block.resnets.0", x, top, top, B, h, w)
+        y = self._resblock("decoder.mid_block.resnets.0", [(x, top)], top, 1e-6, B, h, w)
         self.pool.put(x)
         x = self._vattention(y, top, B, h, w)
         self.pool.put(y)
-        y = self._vres("decoder.mid_block.resnets.1", x, top, top, B, h, w)
+        y = self._resblock("decoder.mid_block.resnets.1", [(x, top)], top, 1e-6, B, h, w)
         self.pool.put(x)
         x, xc = y, top
         # up blocks (vae.py:237-239)
         for j, cin, cout, up in vae_decoder_blocks():
             for k in range(3):
-                y = self._vres(f"decoder.up_blocks.{j}.resnets.{k}", x, cin if k == 0 else cout, cout, B, h, w)
+                y = self._resblock(f"decoder.up_blocks.{j}.resnets.{k}", [(x, cin if k == 0 else cout)], cout, 1e-6, B, h, w)
                 self.pool.put(x)
                 x, xc = y, cout
             if up:
-                rp = f"decoder.up_blocks.{j}.upsamplers.0.conv"
-                y = None
-                if self.act != F32_T and self.net.fold_gathers and B * h * w >= self.net.fold_min_rows_up:
-                    op, _ = self._operand(x, B, h, w, xc)
-                    y, hn, wn = self._conv([(op, xc)], t[f"{rp}.w_up2"], t[f"{rp}.b"], B, h, w, xc, k=3, up=True, want_stats=True, fold_gather=True)
-                    self.pool.put(op)
-                    if y is not None:
-                        h, w = hn, wn
-                if y is None:
-                    if self.act != F32_T:
-                        op, _ = self._operand(x, B, h, w, xc, up=2)
-                        y, h, w = self._conv([(op, xc)], t[f"{rp}.w"], t[f"{rp}.b"], B, 2 * h, 2 * w, xc, k=3, want_stats=True)
-                        self.pool.put(op)
-                    else:
-                        y, h, w = self._conv([(x, xc)], t[f"{rp}.w"], t[f"{rp}.b"], B, h, w, xc, k=3, up=True, want_stats=True)
+                y, h, w = self._upsample_conv(f"decoder.up_blocks.{j}.upsamplers.0.conv", x, xc, B, h, w)
                 self.pool.put(x)
                 x = y
         # GN + SiLU + conv_out 128 -> 3, written straight to NCHW (vae.py:239-241)
@@ -244,67 +150,15 @@ class VAEDecodeProgram(StepProgram):
         self.pool.put(x)
         self._conv([(ao, xc)], t["out.w"], t["out.b"], B, h, w, t["out.b"].shape[0], k=3, out=self.out, out_nchw=True)
         self.pool.put(ao)
-        # shared split-K workspace + one memset of every statistics table at the head of the program
-        need = max([int(lib.sdk_tc_gemm_workspace_bytes(hd)) for hd in self.tc_handles] + [0])
-        self.tc_ws = torch.zeros(max(need, 256), dtype=torch.uint8, device=dev)
-        for hd in self.tc_handles:
-            _lib.check(lib.sdk_tc_gemm_set_workspace(hd, self.tc_ws.data_ptr()))
-        if self.gn_from_sums:
-            self.ops.insert(0, (lib.sdk_zero, (self.stat_arena.data_ptr(), self.stat_used)))
-        self.n_launch = len(self.ops)
 
 
-class VAE(nn.Module):
+class VAE(ProgramModule):
     """Drop-in for the reference ``VAE`` (models/vae/vae.py:244-288), decode path."""
 
     def __init__(self, in_channels: int = 3, z_channels: int = 4):
         super().__init__()
         self.in_channels, self.z_channels = in_channels, z_channels
-        for name, shape in vae_param_spec(in_channels, z_channels):
-            self._register(name, shape)
-        read_knobs(self)
-        self._packed: Dict = {}
-        self._plans: Dict = {}
-        self.register_load_state_dict_post_hook(lambda module, incompatible: module.invalidate())
-
-    def _register(self, name, shape):
-        parts = name.split(".")
-        node = self
-        for p in parts[:-1]:
-            if p not in node._modules:
-                node.add_module(p, _Node())
-            node = node._modules[p]
-        leaf = parts[-1]
-        tns = torch.empty(shape)
-        if "norm" in parts[-2]:
-            tns.fill_(1.0 if leaf == "weight" else 0.0)
-        else:
-            wshape = shape if leaf == "weight" else tuple(getattr(node, "weight").shape)
-            fan_in = 1
-            for d in wshape[1:]:
-                fan_in *= d
-            bound = 1.0 / math.sqrt(fan_in)
-            tns.uniform_(-bound, bound)
-        node.register_parameter(leaf, nn.Parameter(tns, requires_grad=False))
-
-    def invalidate(self):
-        self._packed.clear()
-        self._plans.clear()
-
-    def _apply(self, fn, recurse=True):
-        probe = next(self.parameters())
-        before = (probe.device, probe.dtype, probe.data_ptr())
-        out = super()._apply(fn, recurse)
-        probe = next(self.parameters())
-        if (probe.device, probe.dtype, probe.data_ptr()) != before:
-            self.invalidate()
-        return out
-
-    def set_precision(self, precision: str):
-        if precision not in ("fp32", "bf16"):
-            raise ValueError("precision must be 'fp32' or 'bf16'")
-        self.precision = precision
-        return self
+        self._init_params(vae_param_spec(in_channels, z_channels))
 
     def encode(self, x, noise=None, generator=None):
         raise NotImplementedError("VAE.encode is outside the hot-path scope of this package (SURVEY 8(f)): run the reference encoder")
@@ -325,8 +179,10 @@ class VAE(nn.Module):
         pkey = key + (B, h, w)
         plan = self._plans.get(pkey)
         if plan is None:
-            plan = self._plans[pkey] = _DecodeRunner(VAEDecodeProgram(self, pw, B, h, w), self.use_cuda_graph)
-        return plan(z).to(z.dtype)
+            plan = self._plans[pkey] = GraphRunner(VAEDecodeProgram(self, pw, B, h, w), self.use_cuda_graph)
+        plan.prog.z_in.copy_(z, non_blocking=True)
+        plan.run()
+        return plan.prog.out.clone().to(z.dtype)
 
     @staticmethod
     def from_pretrained(pretrained_path: str, device: str = 'cpu'):
@@ -338,30 +194,3 @@ class VAE(nn.Module):
         sd = load_file(os.path.join(pretrained_path, 'diffusion_pytorch_model.safetensors'), device=device)
         model.load_state_dict(sd, strict=True)
         return model
-
-
-class _DecodeRunner:
-    """Eager on the first call (warm-up), CUDA-graph replay afterwards."""
-
-    def __init__(self, prog: VAEDecodeProgram, use_graph: bool):
-        self.prog, self.use_graph, self.graph, self.calls = prog, use_graph, None, 0
-
-    def __call__(self, z):
-        p = self.prog
-        p.z_in.copy_(z, non_blocking=True)
-        self.calls += 1
-        with torch.cuda.device(p.device):
-            if not self.use_graph:
-                p.launch(p.ops)
-            elif self.graph is None:
-                if self.calls == 1:
-                    p.launch(p.ops)
-                else:
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        p.launch(p.ops)
-                    self.graph = g
-                    g.replay()
-            else:
-                self.graph.replay()
-        return p.out.clone()

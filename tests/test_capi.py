@@ -74,24 +74,24 @@ def test_tune_cache_roundtrip(tmp_path, monkeypatch):
     New measurements are MERGED into the per-user file (never the package's committed cache), keeping other writers' entries."""
     import hashlib
     import json
-    from stable_diffusion_pytorch_b200.unet import StepProgram
+    from stable_diffusion_pytorch_b200.program import LaunchProgram
     f = tmp_path / "user" / "tune.json"
     f.parent.mkdir()
     f.write_text(json.dumps({"NVIDIA B200|2|64|64|320|1|320|3|0|0|0|0|1|1": [160, 1], "NVIDIA B200|1|1|8192|960|1|320|1|0|0|1|0|0|0": [128, 3, 0]}))
-    shipped = hashlib.sha1(open(StepProgram._tune_shipped, "rb").read()).hexdigest()
+    shipped = hashlib.sha1(open(LaunchProgram._tune_shipped, "rb").read()).hexdigest()
     monkeypatch.setenv("SDB200_TC_TUNE_FILE", str(f))
-    monkeypatch.setattr(StepProgram, "_tune_loaded", False)
-    monkeypatch.setattr(StepProgram, "_tune_cache", {})
-    StepProgram._tune_load()
-    assert StepProgram._tune_cache["NVIDIA B200|2|64|64|320|1|320|3|0|0|0|0|1|1"] == (160, 1)      # the user file wins over the shipped one
+    monkeypatch.setattr(LaunchProgram, "_tune_loaded", False)
+    monkeypatch.setattr(LaunchProgram, "_tune_cache", {})
+    LaunchProgram._tune_load()
+    assert LaunchProgram._tune_cache["NVIDIA B200|2|64|64|320|1|320|3|0|0|0|0|1|1"] == (160, 1)      # the user file wins over the shipped one
     # another process added an entry meanwhile: the merge keeps it
     cur = json.loads(f.read_text())
     cur["other-rank"] = [32, 4, 0]
     f.write_text(json.dumps(cur))
-    StepProgram._tune_save("k", (64, 2, 0))
+    LaunchProgram._tune_save("k", (64, 2, 0))
     after = json.loads(f.read_text())
     assert after["k"] == [64, 2, 0] and after["other-rank"] == [32, 4, 0]
-    assert hashlib.sha1(open(StepProgram._tune_shipped, "rb").read()).hexdigest() == shipped       # package file untouched
+    assert hashlib.sha1(open(LaunchProgram._tune_shipped, "rb").read()).hexdigest() == shipped       # package file untouched
 
 
 def test_context_version_helpers():

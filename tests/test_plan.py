@@ -83,13 +83,13 @@ def test_load_rejects_missing_and_foreign_files(tmp_path):
 
 
 def test_slots_encode_floats_and_negative_ints():
-    from stable_diffusion_pytorch_b200.unet import StepProgram
-    s = StepProgram._slots("sdk_gather_row", (0x1000, 20160, 50, 0x2000, -1, 0x3000))
+    from stable_diffusion_pytorch_b200.program import LaunchProgram
+    s = LaunchProgram._slots("sdk_gather_row", (0x1000, 20160, 50, 0x2000, -1, 0x3000))
     assert list(s) == [0x1000, 20160, 50, 0x2000, 0xFFFFFFFFFFFFFFFF, 0x3000]
-    s = StepProgram._slots("sdk_layernorm", (1, 2, 3, 1e-5, 4, 1, 128, 320))
+    s = LaunchProgram._slots("sdk_layernorm", (1, 2, 3, 1e-5, 4, 1, 128, 320))
     assert s[3] == 0x3727C5AC
     with pytest.raises(RuntimeError):
-        StepProgram._slots("sdk_layernorm", (1, 2, 3))
+        LaunchProgram._slots("sdk_layernorm", (1, 2, 3))
 
 
 def test_save_load_roundtrip_and_truncation(tmp_path):
