@@ -65,6 +65,20 @@ int sdk_ddpm_inpaint_step(const float* x, const float* eps_c, const float* eps_u
                           const float* orig, int64_t orig_batch, const uint8_t* mask, const float* noise, float* out,
                           int64_t batch, int64_t channels, int64_t hw, const float* coef_table, int T,
                           const int64_t* t_dev, int64_t t_host, void* stream);
+/* DPM-Solver++(2M) (diffusers' DPMSolverMultistepScheduler, dpmsolver++ / midpoint): the same CFG blend and x0 prediction as
+ * sdk_ddim_step, then x' = A*x + B*x0 + C*(x0 - history), the C term only where the table row flags it (column 7) and
+ * hist_valid != 0 (history is not read otherwise).  history: [n] fp32, the previous step's x0 prediction, replaced by this
+ * step's.  x and out may alias.  The table is the DPMSolverSampler's: it depends on the whole timestep grid. */
+int sdk_dpmpp_step(const float* x, const float* eps_u, const float* eps_c, float cfg_scale, float* history, int hist_valid,
+                   float* out, int64_t n, const float* coef_table, int T, const int64_t* t_dev, int64_t t_host,
+                   int prediction_type, void* stream);
+/* the inpainting loop body of sdk_ddim_inpaint_step with the DPM-Solver++(2M) update of sdk_dpmpp_step;
+ * history: [batch][channels][hw] */
+int sdk_dpmpp_inpaint_step(const float* x, const float* eps_c, const float* eps_u, float cfg_scale,
+                           const float* orig, int64_t orig_batch, const uint8_t* mask, float* out,
+                           int64_t batch, int64_t channels, int64_t hw, const float* coef_table, int T,
+                           const int64_t* t_dev, int64_t t_host, int prediction_type, float* history, int hist_valid,
+                           void* stream);
 /* models/scheduler/ddim.py:46-55 — per-sample timesteps t_dev[batch] */
 int sdk_forward_process(const float* x0, const float* noise, float* out, int64_t batch, int64_t per_sample,
                         const float* coef_table, int T, const int64_t* t_dev, void* stream);

@@ -1,12 +1,12 @@
 """B200-native denoising hot path for dnnhhuy/stable-diffusion-pytorch.
 
 Drop-in replacements for the reference's ``models/unet`` ``UNet.forward(x, timestep, cond)``
-and ``models/scheduler`` samplers, running on hand-written sm_100a CUDA kernels behind a C-ABI
+and ``models/scheduler`` samplers (plus a DPM-Solver++(2M) sampler), running on hand-written sm_100a CUDA kernels behind a C-ABI
 library (include/sdb200.h).  See DESIGN.md / INTEGRATION.md.
 """
-from .scheduler import DDIMSampler, DDPMSampler, x0_from_eps  # noqa: F401
+from .scheduler import DDIMSampler, DDPMSampler, DPMSolverSampler, x0_from_eps  # noqa: F401
 
-__all__ = ["DDIMSampler", "DDPMSampler", "x0_from_eps", "UNet", "VAE", "OpenCLIP", "CLIPTextModel", "CLIPTextConfig", "TextEncoder", "DenoiseLoop", "denoise", "one_step", "img2img", "inpaint"]
+__all__ = ["DDIMSampler", "DDPMSampler", "DPMSolverSampler", "x0_from_eps", "UNet", "VAE", "OpenCLIP", "CLIPTextModel", "CLIPTextConfig", "TextEncoder", "DenoiseLoop", "denoise", "one_step", "img2img", "inpaint"]
 
 
 def __getattr__(name):

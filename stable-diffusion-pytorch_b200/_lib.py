@@ -29,6 +29,8 @@ SIGNATURES = {
     "sdk_ddpm_step": [P, P, P, F32, P, P, I64, P, I32, P, I64, P],
     "sdk_ddim_inpaint_step": [P, P, P, F32, P, I64, P, P, I64, I64, I64, P, I32, P, I64, I32, P],
     "sdk_ddpm_inpaint_step": [P, P, P, F32, P, I64, P, P, P, I64, I64, I64, P, I32, P, I64, P],
+    "sdk_dpmpp_step": [P, P, P, F32, P, I32, P, I64, P, I32, P, I64, I32, P],
+    "sdk_dpmpp_inpaint_step": [P, P, P, F32, P, I64, P, P, I64, I64, I64, P, I32, P, I64, I32, P, I32, P],
     "sdk_forward_process": [P, P, P, I64, I64, P, I32, P, P],
     "sdk_x0_from_eps": [P, P, F32, F32, P, I64, P],
     "sdk_next_timestep": [P, I32, P, P, P],

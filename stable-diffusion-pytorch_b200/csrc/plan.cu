@@ -76,7 +76,8 @@ template <typename... Args> FnEntry entry(const char* name, int (*fn)(Args...), 
 #define E(fn) entry(#fn, &fn)
 const std::vector<FnEntry>& registry() {
     static const std::vector<FnEntry> r = {
-        E(sdk_zero), E(sdk_ddim_step), E(sdk_ddpm_step), E(sdk_ddim_inpaint_step), E(sdk_ddpm_inpaint_step), E(sdk_forward_process), E(sdk_x0_from_eps),
+        E(sdk_zero), E(sdk_ddim_step), E(sdk_ddpm_step), E(sdk_ddim_inpaint_step), E(sdk_ddpm_inpaint_step), E(sdk_dpmpp_step),
+        E(sdk_dpmpp_inpaint_step), E(sdk_forward_process), E(sdk_x0_from_eps),
         E(sdk_next_timestep), E(sdk_gather_row),
         E(sdk_groupnorm_stats), E(sdk_groupnorm_apply), E(sdk_groupnorm_apply_cs), E(sdk_channel_stats), E(sdk_groupnorm_fused),
         E(sdk_groupnorm_cluster), E(sdk_layernorm), E(sdk_softmax_rows), E(sdk_embed_tokens), E(sdk_activation), E(sdk_cast_upsample),

@@ -6,7 +6,7 @@ Per step the reference does: ``latent.repeat(2,...)`` -> UNet -> ``chunk(2)`` ->
 ``sampler.reverse_process`` with three host syncs.  Here a step is a single CUDA-graph replay:
 
     next_timestep (device walk of the host-built grid)  ->  UNet step program (batch 2B, the repeat is
-    folded into the NCHW->NHWC gather)  ->  fused CFG + DDIM/DDPM update, in place on the latent state
+    folded into the NCHW->NHWC gather)  ->  fused CFG + DDIM/DDPM/DPM-Solver++ update, in place on the latent state
 
 so the host enqueues one graph launch per step and never synchronises.  The timestep grid, the
 coefficient tables and all index bookkeeping are the sampler's (bit-exact with the reference).
@@ -20,7 +20,7 @@ import torch
 
 from . import _lib
 from .program import GraphRunner
-from .scheduler import PRED_EPS, PRED_V, DDIMSampler, DDPMSampler, x0_from_eps
+from .scheduler import PRED_EPS, PRED_V, DDIMSampler, DDPMSampler, DPMSolverSampler, x0_from_eps
 from .unet import StepProgram, UNet, same_context, tensor_version
 
 
@@ -34,8 +34,8 @@ class DenoiseLoop:
     def __init__(self, unet: UNet, sampler, batch: int, height: int, width: int, *, do_cfg: bool = True,
                  cfg_scale: float = 7.5, context_len: int = 77, context_batch: Optional[int] = None,
                  device=None, use_cuda_graph: Optional[bool] = None):
-        if not isinstance(sampler, (DDIMSampler, DDPMSampler)):
-            raise TypeError("sampler must be a stable_diffusion_pytorch_b200 DDIMSampler/DDPMSampler")
+        if not isinstance(sampler, (DDIMSampler, DDPMSampler, DPMSolverSampler)):
+            raise TypeError("sampler must be a stable_diffusion_pytorch_b200 DDIMSampler/DDPMSampler/DPMSolverSampler")
         self.unet, self.sampler = unet, sampler
         self.device = torch.device(device) if device is not None else next(unet.parameters()).device
         if self.device.type != "cuda":
@@ -51,6 +51,8 @@ class DenoiseLoop:
         self.latent = self.prog.x_in                         # the loop state IS the UNet's input staging buffer
         with torch.inference_mode(False), torch.no_grad():     # loop state stays writable when built under inference_mode
             self.noise = torch.empty_like(self.latent) if isinstance(sampler, DDPMSampler) else None
+            # DPM-Solver++: the previous step's x0 prediction; the grid's first row is first order and does not read it
+            self.history = torch.empty_like(self.latent) if isinstance(sampler, DPMSolverSampler) else None
             self.counter = torch.zeros(1, dtype=torch.int32, device=self.device)
         self.ts_table = None
         self.tb_table = None
@@ -102,6 +104,17 @@ class DenoiseLoop:
         elif isinstance(s, DDPMSampler):
             _lib.check(lib.sdk_ddpm_step(self.latent.data_ptr(), eps_u, eps_c, self.cfg_scale, self.noise.data_ptr(),
                                          self.latent.data_ptr(), n, self.coef.data_ptr(), s.noise_step, p.t_in.data_ptr(), 0, stream))
+        elif isinstance(s, DPMSolverSampler) and self.inpaint_orig is not None:
+            pred = PRED_V if s.prediction_type == "v_prediction" else PRED_EPS
+            ch = self.latent.shape[1]
+            _lib.check(lib.sdk_dpmpp_inpaint_step(self.latent.data_ptr(), eps_u, eps_c, self.cfg_scale, self.inpaint_orig.data_ptr(),
+                                                  self.inpaint_orig.shape[0], self.inpaint_mask.data_ptr(), self.latent.data_ptr(),
+                                                  self.B, ch, self.H * self.W, self.coef.data_ptr(), s.noise_step, p.t_in.data_ptr(), 0,
+                                                  pred, self.history.data_ptr(), 1, stream))
+        elif isinstance(s, DPMSolverSampler):
+            pred = PRED_V if s.prediction_type == "v_prediction" else PRED_EPS
+            _lib.check(lib.sdk_dpmpp_step(self.latent.data_ptr(), eps_u, eps_c, self.cfg_scale, self.history.data_ptr(), 1,
+                                          self.latent.data_ptr(), n, self.coef.data_ptr(), s.noise_step, p.t_in.data_ptr(), 0, pred, stream))
         elif self.inpaint_orig is not None:
             pred = PRED_V if s.prediction_type == "v_prediction" else PRED_EPS
             ch = self.latent.shape[1]
@@ -116,10 +129,10 @@ class DenoiseLoop:
 
     def export_engine(self, path: str):
         """Engine file of the WHOLE sampling loop for a host without Python (sdk_plan_load; tools/c_host/denoise.c): programs 0-3 of
-        the UNet plan plus program 4 = one sampler step (next timestep -> time-embedding row -> UNet -> CFG + DDIM/DDPM update in
-        place).  Call after ``reset`` (the timestep grid, coefficient and time-embedding tables are baked in as constants).
+        the UNet plan plus program 4 = one sampler step (next timestep -> time-embedding row -> UNet -> CFG + DDIM/DDPM/DPM-Solver++
+        update in place).  Call after ``reset`` (the timestep grid, coefficient and time-embedding tables are baked in as constants).
         Named regions: "x" (the latent state, NCHW fp32), "context", "counter" (int32 grid position: zero it to restart), "out",
-        and "noise" for DDPM."""
+        "noise" for DDPM and "history" (the previous step's x0 prediction) for DPM-Solver++."""
         s, p = self.sampler, self.prog
         if self.ts_table is None:
             raise RuntimeError("export_engine: call reset(latent, context) first (the timestep grid is part of the engine)")
@@ -138,7 +151,11 @@ class DenoiseLoop:
             n = self.latent.numel()
             eps_u = p.out.data_ptr()
             eps_c = p.out.data_ptr() + 4 * n if self.do_cfg else 0
-            if isinstance(s, DDPMSampler):
+            if isinstance(s, DPMSolverSampler):
+                pred = PRED_V if s.prediction_type == "v_prediction" else PRED_EPS
+                p.plan_add(pid, "sdk_dpmpp_step", (self.latent.data_ptr(), eps_u, eps_c, self.cfg_scale, self.history.data_ptr(), 1,
+                                                   self.latent.data_ptr(), n, self.coef.data_ptr(), s.noise_step, p.t_in.data_ptr(), 0, pred))
+            elif isinstance(s, DDPMSampler):
                 p.plan_add(pid, "sdk_ddpm_step", (self.latent.data_ptr(), eps_u, eps_c, self.cfg_scale, self.noise.data_ptr(),
                                                   self.latent.data_ptr(), n, self.coef.data_ptr(), s.noise_step, p.t_in.data_ptr(), 0))
             else:
@@ -150,6 +167,8 @@ class DenoiseLoop:
             extra.append((self.tb_table, 0, ""))
         if self.noise is not None:
             extra.append((self.noise, 2, "noise"))
+        if self.history is not None:
+            extra.append((self.history, 2, "history"))
         p.export_engine(path, extra_regions=extra)
 
     def _prepare(self, context: torch.Tensor):

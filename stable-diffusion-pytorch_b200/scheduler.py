@@ -1,10 +1,12 @@
-"""DDIM / DDPM samplers for the B200 denoising path.
+"""DDIM / DDPM / DPM-Solver++(2M) samplers for the B200 denoising path.
 
 Drop-in for the reference's ``models/scheduler`` classes (reference:
 models/scheduler/ddim.py:7-96, models/scheduler/ddpm.py:10-89): same
 constructor arguments, same attributes (``timesteps``, ``alphas_hat``,
 ``noise_step``, ``inference_steps``, ``prediction_type``) and same method
-names.  ``step`` is an alias of ``reverse_process``.
+names.  ``step`` is an alias of ``reverse_process``.  ``DPMSolverSampler`` adds the
+multistep DPM-Solver++ of order 2 (diffusers' ``DPMSolverMultistepScheduler``,
+"DPM++ 2M") with DDIM's constructor, grid and calling convention.
 
 Split of responsibilities
   * timestep / index bookkeeping stays on the host and is bit-exact with the
@@ -31,7 +33,8 @@ from . import _lib
 COEF_COLS = 8
 _C_S1, _C_S2, _C_SQRT_PREV, _C_DIR, _C_STD = 0, 1, 2, 3, 4          # DDIM
 _P_INV_SQRT_CUR, _P_EPS_COEF, _P_STD = 0, 1, 2                      # DDPM
-_F_SQRT_A, _F_SQRT_1MA = 5, 6                                       # forward_process (both)
+_F_SQRT_A, _F_SQRT_1MA = 5, 6                                       # forward_process (all)
+_D_A, _D_B, _D_C, _D_ORDER2 = 2, 3, 4, 7                            # DPM-Solver++(2M); columns 0-1 are DDIM's
 
 PRED_EPS, PRED_V = 0, 1
 
@@ -98,8 +101,11 @@ class _SamplerBase:
             raise AttributeError(f"{type(self).__name__} has no inference_steps; call _set_inference_steps first")
         return self.noise_step // self.inference_steps
 
+    def _table_key(self):
+        return ()
+
     def _coef_table(self, device, eta: float) -> torch.Tensor:
-        key = (str(device), self._stride(), float(eta), self.prediction_type if hasattr(self, "prediction_type") else "")
+        key = (str(device), self._stride(), float(eta), self.prediction_type if hasattr(self, "prediction_type") else "") + self._table_key()
         tab = self._coef_cache.get(key)
         if tab is None:
             tab = self._build_coef(float(eta)).to(device).contiguous()
@@ -109,6 +115,14 @@ class _SamplerBase:
     def coefficient_table(self, eta: float = 0.0) -> torch.Tensor:
         """Host copy of the per-timestep scalar table the kernel reads ([noise_step, 8] fp32)."""
         return self._build_coef(float(eta))
+
+    @staticmethod
+    def _x0_cols(tab, a_hat):
+        """DDIM's x0-prediction scalars s1 = fp32((1 - a_t)**0.5), s2 = fp32(a_t**0.5), a_t the python double of the fp32
+        table entry (ddim.py:64-66, .item())."""
+        a_list = a_hat.tolist()
+        tab[:, _C_S1] = torch.tensor([(1 - a) ** 0.5 for a in a_list], dtype=torch.float64).to(torch.float32)
+        tab[:, _C_S2] = torch.tensor([a ** 0.5 for a in a_list], dtype=torch.float64).to(torch.float32)
 
     def _forward_cols(self, tab, a_hat):
         tab[:, _F_SQRT_A] = torch.sqrt(a_hat)
@@ -181,8 +195,9 @@ class _SamplerBase:
             return reverse_process(x, timestep, pred)
 
         Note the inpaint loop's own CFG convention: rows ordered [cond ; uncond] and pred = s*(c-u) + c.
-        Both samplers (the reference's inpaint takes sampler='ddim' or 'ddpm', diffusion.py:314-320); with DDPM the update draws
-        fresh N(0,1) noise from torch's global generator like ddpm.py:80 unless ``noise`` is given."""
+        Every sampler (the reference's inpaint takes sampler='ddim' or 'ddpm', diffusion.py:314-320) launches its own update in
+        ``_inpaint_update``; with DDPM the update draws fresh N(0,1) noise from torch's global generator like ddpm.py:80 unless
+        ``noise`` is given, and DPM-Solver++ reads and replaces its history like ``reverse_process``."""
         self._check_cuda(x_t, "inpaint_step")
         x = x_t.contiguous().float()
         b, ch, h, w = x.shape
@@ -207,20 +222,8 @@ class _SamplerBase:
         res = torch.empty_like(x) if out is None else out
         if n == 0:
             return res
-        if isinstance(self, DDPMSampler):
-            if noise is None:
-                noise = torch.randn(x_t.shape, dtype=x_t.dtype, device=x_t.device)
-            nz = noise.to(x.device, torch.float32).contiguous()
-            with torch.cuda.device(x.device):
-                _lib.check(_lib.lib().sdk_ddpm_inpaint_step(
-                    x.data_ptr(), eps_c, eps_u, scale, orig.data_ptr(), orig.shape[0], m8.data_ptr(), nz.data_ptr(), res.data_ptr(), b, ch,
-                    h * w, tab.data_ptr(), self.noise_step, t_ptr, t_host, _lib.current_stream(x.device)))
-            return res
         with torch.cuda.device(x.device):              # launches go to the tensor's device, not the caller's current one
-            _lib.check(_lib.lib().sdk_ddim_inpaint_step(
-                x.data_ptr(), eps_c, eps_u, scale, orig.data_ptr(), orig.shape[0], m8.data_ptr(), res.data_ptr(), b, ch, h * w,
-                tab.data_ptr(), self.noise_step, t_ptr, t_host, PRED_V if self.prediction_type == "v_prediction" else PRED_EPS,
-                _lib.current_stream(x.device)))
+            self._inpaint_update(x_t, x, eps_c, eps_u, scale, orig, m8, res, tab, t_ptr, t_host, noise)
         return res
 
 
@@ -249,9 +252,7 @@ class DDIMSampler(_SamplerBase):
         alphas, a_hat = self._host_tables()
         T, stride = self.noise_step, self._stride()
         tab = torch.zeros(T, COEF_COLS, dtype=torch.float32)
-        a_list = a_hat.tolist()                      # python doubles of the fp32 entries
-        tab[:, _C_S1] = torch.tensor([(1 - a) ** 0.5 for a in a_list], dtype=torch.float64).to(torch.float32)
-        tab[:, _C_S2] = torch.tensor([a ** 0.5 for a in a_list], dtype=torch.float64).to(torch.float32)
+        self._x0_cols(tab, a_hat)
         prev_idx = torch.arange(T) - stride
         a_prev = torch.where(prev_idx >= 0, a_hat[prev_idx.clamp(min=0)], torch.tensor(1.0))
         variance = (1 - a_prev) / (1 - alphas) * (1 - alphas / a_prev)
@@ -261,6 +262,13 @@ class DDIMSampler(_SamplerBase):
         tab[:, _C_STD] = std
         self._forward_cols(tab, a_hat)
         return tab
+
+    def _inpaint_update(self, x_t, x, eps_c, eps_u, scale, orig, m8, res, tab, t_ptr, t_host, noise):
+        b, ch, h, w = x.shape
+        _lib.check(_lib.lib().sdk_ddim_inpaint_step(
+            x.data_ptr(), eps_c, eps_u, scale, orig.data_ptr(), orig.shape[0], m8.data_ptr(), res.data_ptr(), b, ch, h * w,
+            tab.data_ptr(), self.noise_step, t_ptr, t_host, PRED_V if self.prediction_type == "v_prediction" else PRED_EPS,
+            _lib.current_stream(x.device)))
 
     def reverse_process(self, x_t: torch.Tensor, timestep, model_output: torch.Tensor, eta: float = 0.0,
                         *, cfg_scale: Optional[float] = None) -> torch.Tensor:
@@ -348,6 +356,15 @@ class DDPMSampler(_SamplerBase):
         self._forward_cols(tab, a_hat)
         return tab
 
+    def _inpaint_update(self, x_t, x, eps_c, eps_u, scale, orig, m8, res, tab, t_ptr, t_host, noise):
+        b, ch, h, w = x.shape
+        if noise is None:
+            noise = torch.randn(x_t.shape, dtype=x_t.dtype, device=x_t.device)
+        nz = noise.to(x.device, torch.float32).contiguous()
+        _lib.check(_lib.lib().sdk_ddpm_inpaint_step(
+            x.data_ptr(), eps_c, eps_u, scale, orig.data_ptr(), orig.shape[0], m8.data_ptr(), nz.data_ptr(), res.data_ptr(), b, ch,
+            h * w, tab.data_ptr(), self.noise_step, t_ptr, t_host, _lib.current_stream(x.device)))
+
     def reverse_process(self, x_t: torch.Tensor, timestep, model_output: torch.Tensor,
                         *, cfg_scale: Optional[float] = None, noise: Optional[torch.Tensor] = None) -> torch.Tensor:
         """One ancestral DDPM update (reference: ddpm.py:62-82).
@@ -391,6 +408,160 @@ class DDPMSampler(_SamplerBase):
             config = json.load(f)
         return DDPMSampler(noise_step=config["num_train_timesteps"], beta_start=config["beta_start"],
                            beta_end=config["beta_end"], use_cosine_schedule=use_cosine_schedule, device=device)
+
+
+def dpmpp_coefficients(a_path, schedule_steps: Optional[int] = None) -> np.ndarray:
+    """float64 [N, 4] = (A, B, C, order-2 flag) of N DPM-Solver++(2M) steps along a path of N + 1 alpha-bar values.
+
+    diffusers' DPMSolverMultistepScheduler with algorithm_type="dpmsolver++", solver_type="midpoint": with
+    alpha = sqrt(a), sigma = sqrt(1 - a), lambda = log(alpha) - log(sigma) and h = lambda_t - lambda_s for step s -> t,
+        x_t = A*x_s + B*m0 + C*(m0 - m1),   A = sigma_t/sigma_s,  B = -alpha_t*expm1(-h),  C = B/(2r),
+    r = (lambda_s - lambda_prev)/h, m0 / m1 the x0 predictions at s and at the step before.  A step to a = 1 (sigma = 0, the
+    last step of a sampling grid) has A = 0, B = 1: it returns m0.  Steps are first order (C = 0, flag 0) on the first step,
+    the last step, and the second-to-last step when the schedule has fewer than 15 steps.  ``schedule_steps`` is the length of
+    the whole schedule (default N): a path that is the tail of a longer schedule (img2img strength) counts the whole schedule,
+    as diffusers does when it starts a pipeline part-way through its timesteps."""
+    a = np.asarray(a_path, dtype=np.float64)
+    n = len(a) - 1
+    short = (n if schedule_steps is None else schedule_steps) < 15
+    alpha, sigma = np.sqrt(a), np.sqrt(1.0 - a)
+    with np.errstate(divide="ignore"):
+        lam = np.log(alpha) - np.log(sigma)                  # +inf where sigma == 0
+    out = np.zeros((n, 4), dtype=np.float64)
+    for i in range(n):
+        if sigma[i + 1] == 0.0:
+            out[i, 0], out[i, 1] = 0.0, 1.0
+        else:
+            h = lam[i + 1] - lam[i]
+            out[i, 0] = sigma[i + 1] / sigma[i]
+            out[i, 1] = -alpha[i + 1] * np.expm1(-h)
+        order2 = 0 < i < n - 1 and not (i == n - 2 and short)
+        if order2:
+            r = (lam[i] - lam[i - 1]) / (lam[i + 1] - lam[i])
+            out[i, 2] = out[i, 1] / (2.0 * r)
+            out[i, 3] = 1.0
+    return out
+
+
+class DPMSolverSampler(_SamplerBase):
+    """Multistep DPM-Solver++ of order 2 ("DPM++ 2M"; diffusers' DPMSolverMultistepScheduler defaults: dpmsolver++,
+    midpoint, lower_order_final, final sigma zero) on DDIM's timestep grid, commonly run at 20-25 steps.
+
+    Same constructor, ``from_config``, grid (bit for bit), ``set_strength`` and ``forward_process`` as ``DDIMSampler``; the
+    final step goes to alpha-bar = 1 and returns the x0 prediction.  The update needs the previous step's x0 prediction: the
+    sampler keeps it in a device tensor per shape and device.  A host flag says whether that history belongs to the current
+    sequence; ``_set_inference_steps``, ``set_strength``, ``reset()`` and a change of shape or device clear it, so a sequence
+    that starts anywhere takes a first-order step instead of reading stale history.  The coefficient table depends on the
+    whole grid; a timestep off the grid poisons the update with NaN, like an out-of-range one."""
+    _timestep_offset = 1
+
+    def __init__(self, noise_step: int = 1000, beta_start: float = 0.00085, beta_end: float = 0.012,
+                 use_cosine_schedule: bool = False, device: str = 'cpu', prediction_type: str = "epsilon"):
+        self._init_tables(noise_step, beta_start, beta_end, use_cosine_schedule, device)
+        self.inference_steps = self.noise_step
+        self.prediction_type = prediction_type
+        self._hist, self._hist_valid = None, False
+
+    def _sample_timestep(self, n, device):
+        return torch.randint(low=0, high=self.noise_step, size=(n,), device=device)
+
+    def reset(self):
+        """Forget the history: the next step is first order."""
+        self._hist_valid = False
+
+    def _set_inference_steps(self, inference_steps=50):
+        super()._set_inference_steps(inference_steps)
+        self.reset()
+
+    def set_strength(self, strength: float = 0.8):
+        super().set_strength(strength)
+        self.reset()
+
+    def _history(self, x: torch.Tensor):
+        """-> (history tensor for x's shape and device, hist_valid for this step).  The caller marks the history valid
+        (``_hist_valid = True``) once the step that fills it has been launched."""
+        if self._hist is None or self._hist.shape != x.shape or self._hist.device != x.device:
+            with torch.inference_mode(False), torch.no_grad():
+                self._hist = torch.empty_like(x)
+            self._hist_valid = False
+        return self._hist, int(self._hist_valid)
+
+    def _inpaint_update(self, x_t, x, eps_c, eps_u, scale, orig, m8, res, tab, t_ptr, t_host, noise):
+        b, ch, h, w = x.shape
+        hist, valid = self._history(x)
+        _lib.check(_lib.lib().sdk_dpmpp_inpaint_step(
+            x.data_ptr(), eps_c, eps_u, scale, orig.data_ptr(), orig.shape[0], m8.data_ptr(), res.data_ptr(), b, ch, h * w,
+            tab.data_ptr(), self.noise_step, t_ptr, t_host, PRED_V if self.prediction_type == "v_prediction" else PRED_EPS,
+            hist.data_ptr(), valid, _lib.current_stream(x.device)))
+        self._hist_valid = True
+
+    def _table_key(self):
+        return (self.inference_steps,) + tuple(self.timesteps.tolist())
+
+    def _build_coef(self, eta: float = 0.0) -> torch.Tensor:
+        """[noise_step, 8] fp32: columns 0-1 and 5-6 are DDIM's (bit for bit); on the rows of the current grid t_0 > ... > t_N-1,
+        columns 2-4 = A, B, C and 7 = the order-2 flag of ``dpmpp_coefficients`` along alpha-bar[t_0], ..., alpha-bar[t_N-1], 1.0,
+        computed in float64 and rounded to fp32 once; the lower-order-final rule counts the whole ``inference_steps`` schedule, so
+        a ``set_strength`` tail keeps the flags it has in the full grid except on its first row.  Other rows are NaN in columns 2-4."""
+        _, a_hat = self._host_tables()
+        T = self.noise_step
+        tab = torch.zeros(T, COEF_COLS, dtype=torch.float32)
+        self._x0_cols(tab, a_hat)
+        self._forward_cols(tab, a_hat)
+        tab[:, _D_A:_D_C + 1] = float("nan")
+        grid = [int(t) for t in self.timesteps.tolist()]
+        if any(t < 0 or t >= T for t in grid):
+            raise ValueError(f"timestep grid {grid} outside [0, {T})")
+        a_path = a_hat.to(torch.float64)[grid].tolist() + [1.0]
+        k = torch.from_numpy(dpmpp_coefficients(a_path, self.inference_steps)).to(torch.float32)
+        rows = torch.tensor(grid, dtype=torch.int64)
+        tab[rows, _D_A], tab[rows, _D_B], tab[rows, _D_C], tab[rows, _D_ORDER2] = k[:, 0], k[:, 1], k[:, 2], k[:, 3]
+        return tab
+
+    def reverse_process(self, x_t: torch.Tensor, timestep, model_output: torch.Tensor, *,
+                        cfg_scale: Optional[float] = None) -> torch.Tensor:
+        """One DPM-Solver++(2M) update from ``timestep`` to the next point of the grid (alpha-bar = 1 after the last).
+
+        Calling convention of ``DDIMSampler.reverse_process``: host or device timestep, no host sync, and with ``cfg_scale``
+        given ``model_output`` is the (2B, ...) UNet output ordered [uncond ; cond], blended as u + s*(c-u) in the same kernel.
+        Reads the previous step's x0 prediction from the sampler's history and replaces it with this step's."""
+        self._check_cuda(x_t, "reverse_process")
+        if self.prediction_type not in ("epsilon", "v_prediction"):
+            raise ValueError(f"unknown prediction_type {self.prediction_type!r}")
+        x = x_t.contiguous().float()
+        mo = model_output.to(x.device, torch.float32).contiguous()
+        n = x.numel()
+        if cfg_scale is None:
+            if mo.shape != x.shape:
+                raise RuntimeError(f"model_output {tuple(mo.shape)} vs x_t {tuple(x.shape)}")
+            eps_u, eps_c, scale = mo.data_ptr(), 0, 0.0
+        else:
+            if mo.shape[0] != 2 * x.shape[0] or mo.shape[1:] != x.shape[1:]:
+                raise RuntimeError(f"CFG model_output must be (2B, ...) = {(2 * x.shape[0],) + tuple(x.shape[1:])}, got {tuple(mo.shape)}")
+            eps_u, eps_c, scale = mo.data_ptr(), mo.data_ptr() + n * 4, float(cfg_scale)
+        tab = self._coef_table(x.device, 0.0)
+        t_ptr, t_host, keep = self._timestep_args(timestep, x.device)
+        out = torch.empty_like(x)
+        if n == 0:
+            return out
+        hist, valid = self._history(x)
+        with torch.cuda.device(x.device):              # launches go to the tensor's device, not the caller's current one
+            _lib.check(_lib.lib().sdk_dpmpp_step(
+                x.data_ptr(), eps_u, eps_c, scale, hist.data_ptr(), valid, out.data_ptr(), n, tab.data_ptr(), self.noise_step,
+                t_ptr, t_host, PRED_V if self.prediction_type == "v_prediction" else PRED_EPS, _lib.current_stream(x.device)))
+        self._hist_valid = True
+        return out
+
+    step = reverse_process
+
+    @staticmethod
+    def from_config(cfg_path: str, use_cosine_schedule: bool = False, device: str = 'cpu'):
+        """Reads <cfg_path>/scheduler_config.json like DDIMSampler.from_config."""
+        with open(os.path.join(cfg_path, "scheduler_config.json"), 'r') as f:
+            config = json.load(f)
+        return DPMSolverSampler(noise_step=config["num_train_timesteps"], beta_start=config["beta_start"],
+                                beta_end=config["beta_end"], use_cosine_schedule=use_cosine_schedule, device=device,
+                                prediction_type=config.get("prediction_type", "epsilon"))
 
 
 def x0_from_eps(latent: torch.Tensor, pred_noise: torch.Tensor, alpha_T: float = 0.0047 ** 0.5,
