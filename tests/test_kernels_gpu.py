@@ -1,7 +1,9 @@
 """GPU kernel-level parity: every C-ABI kernel against a plain PyTorch fp32 reference of the same op
 (TF32 disabled) on seeded inputs.  Tolerances: fp32 kernels 2e-5 rel-L2; bf16-operand kernels are
 compared on bf16-ROUNDED inputs with fp32 reference math, so only accumulation order and the final
-output rounding differ (<= 4e-3 for bf16 outputs, <= 2e-5 for fp32 outputs)."""
+output rounding differ (<= 4e-3 for bf16 outputs, <= 2e-5 for fp32 outputs).  The causal attention, row softmax, token embedding,
+activation and VAE-attention GEMM tests compare with float64 references, element- or row-wise where a global norm could hide one bad
+row."""
 import ctypes as C
 import math
 
@@ -126,6 +128,9 @@ TC_CASES = [
     ("ws_geglu_L0", 1, 1, 8192, 320, 2560, 1, None, False, True, BF16_T, 0, 160, 1),
     ("ws_qkv_L0", 1, 1, 8192, 320, 960, 1, None, False, False, BF16_T, 0, 160, 1),
     ("ws_lin_L1_bn64", 1, 1, 16384, 640, 1920, 1, None, False, False, BF16_T, 0, 64, 1),
+    # text encoders (OpenCLIP-H, batch 2 x 77 tokens): q|k|v projection and fc2 + residual
+    ("clip_qkv", 1, 1, 154, 1024, 3072, 1, None, False, False, BF16_T, 0, 0, 0),
+    ("clip_fc2_res", 1, 1, 154, 4096, 1024, 1, None, True, False, F32_T, 0, 0, 0),
 ]
 
 
@@ -260,14 +265,106 @@ def test_tc_gemm_two_segments(dev):
     assert rel_l2(out, want) < 2e-5
 
 
+def bits(t):
+    """The raw bits of a bf16 / fp32 tensor: equality that tells -0 from 0."""
+    return t.view(torch.int16 if t.element_size() == 2 else torch.int32)
+
+
+# causal self-attention of the text encoders (clip.py:120-121): (B, heads, S, S, D, "causal").  S crosses the fp32 kernel's 32-key
+# tiles and 64-row blocks and the tcgen05 kernel's 32-key streams, 64-key tiles and 128-row query tiles; every D at S = 77 and 129
+CAUSAL_CASES = [(1, 4, 1, 1, 64), (2, 4, 20, 20, 40), (1, 16, 33, 33, 80), (2, 4, 64, 64, 160), (1, 16, 65, 65, 64),
+                (2, 16, 77, 77, 40), (2, 16, 77, 77, 64), (1, 16, 77, 77, 80), (2, 16, 77, 77, 160), (1, 4, 128, 128, 80),
+                (2, 4, 129, 129, 40), (2, 4, 129, 129, 64), (1, 4, 129, 129, 80), (2, 16, 129, 129, 160), (2, 16, 300, 300, 64)]
+CAUSAL_PARAMS = [pytest.param(c + ("causal",), id=f"causal-B{c[0]}-h{c[1]}-S{c[2]}-D{c[4]}") for c in CAUSAL_CASES]
+# prefix split points: the 32-key streams / tiles, the 64-key tiles and 64-row blocks, the 128-row query tiles
+CAUSAL_SPLITS = (1, 31, 32, 33, 63, 64, 65, 127, 128, 129)
+
+
+def causal_reference(qkv, B, Hh, S, D):
+    """softmax(Q K^T / sqrt(D) + mask) V in float64, mask = -inf where key > query; qkv [B][S][q|k|v] -> [B][S][heads * D]."""
+    t = qkv.double().view(B, S, 3, Hh, D).permute(2, 0, 3, 1, 4)
+    s = (t[0] @ t[1].transpose(-1, -2)) * D ** -0.5
+    s = s.masked_fill(torch.ones((S, S), dtype=torch.bool, device=qkv.device).triu(1), float("-inf"))
+    return (torch.softmax(s, -1) @ t[2]).permute(0, 2, 1, 3).reshape(B, S, Hh * D)
+
+
+def check_causal_attention(dev, B, Hh, S, D, kernel):
+    """Causal self-attention of the fp32 kernel (sdk_attention_f32_ex, causal = 1) or the tcgen05 kernel (sdk_attention_tc_set_causal)
+    on a q|k|v buffer with per-batch K / V: against float64 globally and row by row, and prefix-invariant bit for bit (rows < p do
+    not see keys >= p).  The tcgen05 handle must give the non-causal result again once the mask is switched off."""
+    lib = _lib.lib()
+    Cc = Hh * D
+    dt = torch.float32 if kernel == "f32" else torch.bfloat16
+    qkv = gen((B, S, 3 * Cc), 131, dev).to(dt)
+    buf = torch.empty_like(qkv)
+    out = torch.full((B, S, Cc), float("nan"), device=dev, dtype=dt)
+    st = (3 * Cc, S * 3 * Cc)
+    args = (buf.data_ptr(), *st, buf.data_ptr() + Cc * qkv.element_size(), *st, buf.data_ptr() + 2 * Cc * qkv.element_size(), *st,
+            out.data_ptr(), Cc, S * Cc, B, Hh, S, S, D, float(D ** -0.5))
+    h = C.c_void_p()
+    if kernel == "tc":
+        _lib.check(lib.sdk_attention_tc_create(*args, C.byref(h)))
+        _lib.check(lib.sdk_attention_tc_set_causal(h, 1))
+
+    def run(x):
+        buf.copy_(x)
+        out.fill_(float("nan"))
+        for _ in range(2):
+            if kernel == "tc":
+                _lib.check(lib.sdk_attention_tc_launch(h, stream()))
+            else:
+                _lib.check(lib.sdk_attention_f32_ex(*args, 1, stream()))
+        torch.cuda.synchronize()
+        return out.clone()
+
+    try:
+        y = run(qkv)
+        assert not torch.isnan(y.float()).any()
+        want = causal_reference(qkv, B, Hh, S, D)
+        e = rel_l2(y, want)
+        dy, w4 = (y.double() - want).view(B, S, Hh, D), want.view(B, S, Hh, D)
+        rows = dy.norm(dim=-1) / w4.norm(dim=-1)                       # [B][S][heads]
+        worst, at = float(rows.max()), int(rows.argmax())
+        print(f"causal attention {kernel} B{B} heads{Hh} S{S} D{D}: rel-L2 {e:.2e}, worst (b, row, head) {worst:.2e} "
+              f"at {(at // (S * Hh), at // Hh % S, at % Hh)}")
+        assert e < (2e-5 if kernel == "f32" else 8e-3)
+        assert worst < (1e-4 if kernel == "f32" else 2e-2)
+        fresh = gen((B, S, 3 * Cc), 132, dev).to(dt)
+        for p in CAUSAL_SPLITS:
+            if p >= S:
+                break
+            alt = qkv.clone()
+            alt[:, p:, Cc:] = fresh[:, p:, Cc:]                    # new keys and values from position p on
+            y2 = run(alt)
+            assert torch.equal(bits(y2[:, :p]), bits(y[:, :p])), f"rows < {p} read keys >= {p}"
+            changed = (bits(y2[:, p]) != bits(y[:, p])).view(B, Hh, D).any(-1)
+            assert bool(changed.all()), f"row {p} does not read key {p}"
+        if kernel == "tc":
+            _lib.check(lib.sdk_attention_tc_set_causal(h, 0))
+            y0 = run(qkv)
+            t = qkv.double().view(B, S, 3, Hh, D).permute(2, 0, 3, 1, 4)
+            full = (torch.softmax((t[0] @ t[1].transpose(-1, -2)) * D ** -0.5, -1) @ t[2]).permute(0, 2, 1, 3).reshape(B, S, Cc)
+            e0 = rel_l2(y0, full)
+            print(f"  same handle, causal off: rel-L2 {e0:.2e} vs non-causal")
+            assert e0 < 8e-3
+    finally:
+        if kernel == "tc":
+            lib.sdk_attention_tc_destroy(h)
+
+
 ATT_CASES = [(2, 8, 1024, 1024, 40), (2, 8, 256, 256, 160), (1, 8, 1024, 77, 80), (2, 5, 576, 576, 64),
              (2, 8, 64, 77, 160), (1, 8, 100, 77, 40), (2, 20, 144, 144, 64)]
 
 
-@pytest.mark.parametrize("case", ATT_CASES)
+@pytest.mark.parametrize("case", ATT_CASES + CAUSAL_PARAMS)
 @pytest.mark.parametrize("mode", ["f32", "bf16"])
 def test_attention(dev, case, mode):
-    B, Hh, Sq, Sk, D = case
+    B, Hh, Sq, Sk, D = case[:5]
+    if len(case) > 5:
+        if mode == "bf16":
+            pytest.skip("sdk_attention_bf16 has no causal path: bf16 causal attention runs on the tcgen05 kernel")
+        check_causal_attention(dev, B, Hh, Sq, D, "f32")
+        return
     lib = _lib.lib()
     Cc = Hh * D
     dt = torch.float32 if mode == "f32" else torch.bfloat16
@@ -304,10 +401,13 @@ ATT_TC_CASES = [(2, 8, 4096, 4096, 40), (1, 8, 1024, 77, 40), (2, 5, 2304, 2304,
                 (2, 8, 64, 77, 160), (16, 8, 1024, 1024, 80), (3, 8, 200, 333, 80), (1, 8, 100, 130, 160)]
 
 
-@pytest.mark.parametrize("case", ATT_TC_CASES)
+@pytest.mark.parametrize("case", ATT_TC_CASES + CAUSAL_PARAMS)
 def test_attention_tc(dev, case):
     """tcgen05 flash attention (head_dim 40 / 64 / 80 / 160) vs fp32 softmax(QK^T/sqrt(D))V on the bf16-rounded inputs."""
-    B, Hh, Sq, Sk, D = case
+    B, Hh, Sq, Sk, D = case[:5]
+    if len(case) > 5:
+        check_causal_attention(dev, B, Hh, Sq, D, "tc")
+        return
     lib = _lib.lib()
     Cc = Hh * D
     dt = torch.bfloat16
@@ -723,7 +823,7 @@ def test_linear_layernorm_unsupported_width(dev):
     assert lib.sdk_linear_ln_create(C.byref(d), C.byref(h)) == -3
 
 
-@pytest.mark.parametrize("C_", [320, 640, 1280, 768])
+@pytest.mark.parametrize("C_", [320, 640, 1280, 768, 256, 1024])
 def test_layernorm(dev, C_):
     lib = _lib.lib()
     x = gen((1000, C_), 51, dev) * 3 + 1
@@ -770,3 +870,201 @@ def test_cast_upsample_im2col_nchw(dev):
     nhwc = torch.empty((2, 64, 4), device=dev)
     _lib.check(lib.sdk_nchw_to_nhwc(lat.data_ptr(), nhwc.data_ptr(), 1, 2, 4, 64, stream()))
     assert torch.equal(nhwc, lat.repeat(2, 1, 1, 1).permute(0, 2, 3, 1).reshape(2, 64, 4))
+
+
+# ------------------------------------------------------------------------------------------------
+# row softmax of the VAE attention (vae.py:90), the text encoders' token embedding and activations (clip.py:114,130)
+# ------------------------------------------------------------------------------------------------
+FLT_MIN = 2.0 ** -126                                   # smallest normal fp32: below it the kernel's exp2 / product are subnormal
+
+
+@pytest.mark.parametrize("rows,cols", [(300, 4), (300, 64), (300, 1020), (300, 1024), (200, 4096), (64, 9216), (24, 16384)])
+def test_softmax_rows(dev, rows, cols):
+    """sdk_softmax_rows vs float64 softmax of the same fp32 scores: logits spanning +-80 in the exp2 domain, a row with one dominant
+    entry, a row of equal values.  Every element within 1e-5 relative (absolute FLT_MIN where fp32 underflows), every row sums to 1;
+    the bf16 output is the fp32 output rounded."""
+    lib = _lib.lib()
+    scale = 512 ** -0.5
+    sl2 = float(np.float32(np.float32(scale) * np.float32(1.4426950408889634)))      # the kernel's fp32 scale * log2(e)
+    g = torch.Generator().manual_seed(141)
+    x = (torch.rand((rows, cols), generator=g, dtype=torch.float64) * 160 - 80) / sl2
+    x[1] = torch.randn(cols, generator=g, dtype=torch.float64) / sl2
+    x[1, cols // 3] += 80 / sl2                                                     # one entry 2^80 above the rest
+    x[2] = 3.0                                                                      # all equal: 1 / cols
+    x = x.float().to(dev)
+    want = torch.softmax(x.double() * (sl2 * math.log(2.0)), dim=-1)
+    y = torch.full((rows, cols), float("nan"), device=dev)
+    yb = torch.full((rows, cols), float("nan"), device=dev, dtype=torch.bfloat16)
+    for out, odt in ((y, F32_T), (yb, BF16_T)):
+        _lib.check(lib.sdk_softmax_rows(x.data_ptr(), out.data_ptr(), odt, rows, cols, scale, stream()))
+    torch.cuda.synchronize()
+    err = (y.double() - want).abs()
+    worst = float(((err - FLT_MIN).clamp_min(0) / want).max())
+    row_sum = float((y.double().sum(-1) - 1).abs().max())
+    print(f"softmax rows={rows} cols={cols}: worst element rel err {worst:.2e}, worst |row sum - 1| {row_sum:.2e}")
+    assert not torch.isnan(y).any()
+    assert bool((err <= 1e-5 * want + FLT_MIN).all())
+    assert row_sum <= 1e-5
+    assert float((y[2].double() - 1.0 / cols).abs().max()) <= 1e-5 / cols
+    assert torch.equal(bits(yb), bits(y.bfloat16()))
+
+
+def test_softmax_rows_contract(dev):
+    lib = _lib.lib()
+    buf = torch.zeros(64, device=dev)
+    p = buf.data_ptr()
+    assert lib.sdk_softmax_rows(p, p, F32_T, 1, 6, 1.0, stream()) == -1               # cols % 4 != 0
+    assert lib.sdk_softmax_rows(p, p, F32_T, 1, 16388, 1.0, stream()) == -1           # wider than 16384
+    assert lib.sdk_softmax_rows(p, p, 2, 1, 16, 1.0, stream()) == -1                  # no such output type
+    assert lib.sdk_softmax_rows(p, p, F32_T, 0, 16, 1.0, stream()) == 0               # no rows: nothing to do
+
+
+EMBED_CASES = [(77, 1, 256), (77, 2, 768), (77, 2, 1024), (20, 1, 1024), (20, 2, 256), (20, 2, 768),
+               (77, 32, 1024)]                                  # 2464 rows x 256 float4: more than one pass of the capped grid
+
+
+@pytest.mark.parametrize("S,B,C_", EMBED_CASES)
+def test_embed_tokens(dev, S, B, C_):
+    """sdk_embed_tokens == tok[ids] + pos[r % S] exactly; ids outside [0, vocab) are clamped to the table."""
+    lib = _lib.lib()
+    vocab, rows = 1000, B * S
+    tok = gen((vocab, C_), 151, dev)
+    pos = gen((77, C_), 152, dev)                               # the encoders' max_len positions; S of them are read
+    g = torch.Generator().manual_seed(153)
+    ids = torch.randint(0, vocab, (B, S), generator=g, dtype=torch.int64)
+    ids.view(-1)[:5] = torch.tensor([0, vocab - 1, -1, vocab, 2 ** 40])
+    ids.view(-1)[-3:] = torch.tensor([-(2 ** 40), vocab - 1, 0])
+    ids = ids.to(dev)
+    out = torch.full((B, S, C_), float("nan"), device=dev)
+    _lib.check(lib.sdk_embed_tokens(ids.data_ptr(), tok.data_ptr(), pos.data_ptr(), out.data_ptr(), rows, S, C_, vocab, stream()))
+    torch.cuda.synchronize()
+    want = tok[ids.clamp(0, vocab - 1)] + pos[:S][None]
+    assert torch.equal(bits(out), bits(want))
+    if B == 32:
+        sms = torch.cuda.get_device_properties(dev).multi_processor_count
+        assert rows * C_ // 4 > sms * 8 * 256, "the grid-stride loop must run more than once"
+
+
+@pytest.mark.parametrize("n", [4, 1020, 1 << 21])              # 2^21 / 4 float4 > 8 CTAs x 256 threads per SM: grid-stride
+@pytest.mark.parametrize("kind", [1, 2], ids=["gelu", "quickgelu"])
+def test_activation(dev, kind, n):
+    """sdk_activation (1: exact-erf GELU, 2: QuickGELU x * sigmoid(1.702 x)) vs float64 on a dense grid over [-30, 30] plus 0, -0,
+    +-1e4: absolute error <= 1e-6 * max(1, |x|), never NaN; the bf16 output is the fp32 output rounded."""
+    lib = _lib.lib()
+    x = torch.cat([torch.tensor([0.0, -0.0, 1e4, -1e4], dtype=torch.float64), torch.linspace(-30, 30, n - 4, dtype=torch.float64)])
+    x = x.float().to(dev)
+    xd = x.double()
+    want = 0.5 * xd * torch.special.erfc(-xd / math.sqrt(2.0)) if kind == 1 else xd * torch.sigmoid(1.702 * xd)
+    y = torch.full((n,), float("nan"), device=dev)
+    yb = torch.full((n,), float("nan"), device=dev, dtype=torch.bfloat16)
+    for out, odt in ((y, F32_T), (yb, BF16_T)):
+        _lib.check(lib.sdk_activation(x.data_ptr(), out.data_ptr(), odt, n, kind, stream()))
+    torch.cuda.synchronize()
+    err = (y.double() - want).abs() / xd.abs().clamp_min(1.0)
+    print(f"activation kind {kind} n={n}: worst abs err / max(1, |x|) {float(err.max()):.2e}")
+    assert not torch.isnan(y).any()
+    assert float(err.max()) <= 1e-6
+    assert float(y[3]) == 0.0                                   # x = -1e4: -0 or 0 (QuickGELU's exp overflows to inf)
+    assert torch.equal(bits(yb), bits(y.bfloat16()))
+
+
+# ------------------------------------------------------------------------------------------------
+# the VAE mid-block attention's three GEMMs (vae.py:85-91), each on its own bf16-rounded operands
+# ------------------------------------------------------------------------------------------------
+def vae_attention_operands(dev, S, Cc=512):
+    """Operands of one sample's attention GEMMs.  The token, q and k buffers hold two samples, and sample 1 is read through its
+    slice pointer as in the per-sample loop.  P is a row softmax, so the bias of P V is a visible part of the output."""
+    g = torch.Generator().manual_seed(161)
+
+    def r(*shape, s=1.0):
+        return (torch.randn(shape, generator=g) * s).to(dev)
+
+    ops = dict(tokens=r(2 * S, Cc), wv=r(Cc, Cc, s=Cc ** -0.5), q=r(2 * S, Cc), k=r(2 * S, Cc),
+               p=torch.softmax(r(S, S, s=2.0), -1), vT=r(Cc, S), bv=r(Cc, s=0.1))
+    return ops
+
+
+def vae_attention_stage(ops, stage, S, Cc=512):
+    """(A [M][K], B operand [N][K] row-major, bias, M, N, K, output rows offset) of one stage: V^T = W_v tokens^T (N = S),
+    scores = q k^T (fp32 [S][S]), out = P V + b_v (K = S, written to rows S..2S of the batch's output)."""
+    if stage == "vT":
+        return ops["wv"], ops["tokens"][S:], None, Cc, S, Cc, 0
+    if stage == "scores":
+        return ops["q"][S:], ops["k"][S:], None, S, S, Cc, 0
+    return ops["p"], ops["vT"], ops["bv"], S, Cc, S, S
+
+
+VAE_ATT_STAGES = ([pytest.param("vT", (0, 0), id="vT-auto"), pytest.param("scores", (0, 0), id="scores-auto")] +
+                  [pytest.param("pv", t, id=f"pv-bn{t[0]}-sp{t[1]}") for t in ((0, 0), (64, 1), (128, 2), (256, 4))])
+
+
+@pytest.mark.parametrize("S", [64, 128, 576, 4096, 9216])
+@pytest.mark.parametrize("stage,tiling", VAE_ATT_STAGES)
+def test_tc_gemm_vae_attention(dev, stage, tiling, S):
+    """The tensor-core GEMMs of the VAE attention with an ACTIVATION as the row-major B operand (w_kmajor = 0, w_const = 0, as
+    _emit_tc_conv sets them for w_rowmajor) vs float64 on the bf16 operands; P V also with forced (block_n, split-K) tilings."""
+    lib = _lib.lib()
+    ops = {k: v.bfloat16() if k != "bv" else v for k, v in vae_attention_operands(dev, S).items()}
+    a, w, bias, M, N, K, row0 = vae_attention_stage(ops, stage, S)
+    odt = F32_T if stage == "scores" else BF16_T
+    out_all = torch.full((row0 + M, N), float("nan"), device=dev, dtype=torch.float32 if odt == F32_T else torch.bfloat16)
+    out = out_all[row0:]
+    d = TcGemmDesc()
+    d.w_kmajor, d.w_const = 0, 0
+    d.a[0], d.w[0], d.C[0], d.ksize[0], d.nseg = a.data_ptr(), w.data_ptr(), K, 1, 1
+    d.B, d.H, d.W, d.N = 1, 1, M, N
+    d.bias = bias.data_ptr() if bias is not None else 0
+    d.out, d.out_dtype = out.data_ptr(), odt
+    d.block_n, d.splits = tiling
+    h = C.c_void_p()
+    _lib.check(lib.sdk_tc_gemm_create(C.byref(d), C.byref(h)))
+    info = (C.c_int * 11)()
+    _lib.check(lib.sdk_tc_gemm_info(h, info, 11))
+    ws = torch.zeros(max(int(lib.sdk_tc_gemm_workspace_bytes(h)), 256), dtype=torch.uint8, device=dev)
+    _lib.check(lib.sdk_tc_gemm_set_workspace(h, ws.data_ptr()))
+    for _ in range(2):                                    # twice: split-K tickets must re-arm
+        _lib.check(lib.sdk_tc_gemm_launch(h, stream()))
+    torch.cuda.synchronize()
+    lib.sdk_tc_gemm_destroy(h)
+    want = a.double() @ w.double().t()
+    if bias is not None:
+        want = want + bias.double()
+    e = rel_l2(out, want)
+    print(f"VAE attention {stage} S={S} M={M} N={N} K={K}: block_n={info[0]} splits={info[1]} grid=({info[2]},{info[3]}) "
+          f"kernel={('plain', 'persistent', 'persistent weight-stationary')[info[10]]} rel-L2 {e:.2e}")
+    assert not torch.isnan(out.float()).any()
+    assert e < (2e-5 if odt == F32_T else 4e-3)
+    if row0:
+        assert torch.isnan(out_all[:row0].float()).all(), "wrote outside the sample's rows"
+    if tiling != (0, 0):                                  # the forced split count, as the library rounds it to whole k-blocks
+        kb = K // 64
+        per = -(-kb // min(tiling[1], kb))
+        assert info[0] == tiling[0] and info[1] == -(-kb // per)
+
+
+@pytest.mark.parametrize("S", [64, 576, 4096])
+@pytest.mark.parametrize("stage", ["vT", "scores", "pv"])
+def test_conv_gemm_f32_vae_attention(dev, stage, S):
+    """The same three products in the fp32 mode (sdk_conv_gemm_f32, the B operand a plain [N][K] matrix) vs float64."""
+    lib = _lib.lib()
+    ops = vae_attention_operands(dev, S)
+    a, w, bias, M, N, K, row0 = vae_attention_stage(ops, stage, S)
+    out_all = torch.full((row0 + M, N), float("nan"), device=dev)
+    out = out_all[row0:]
+    p = ConvParams()
+    p.src0, p.src1, p.C0, p.C1 = a.data_ptr(), 0, K, 0
+    p.weight, p.bias = w.data_ptr(), (bias.data_ptr() if bias is not None else 0)
+    p.tbias, p.tb_stride, p.residual, p.out = 0, 0, 0, out.data_ptr()
+    p.B, p.Hin, p.Win, p.Hout, p.Wout = 1, 1, M, 1, M
+    p.ksize, p.stride, p.upsample, p.N = 1, 1, 0, N
+    p.in_dtype, p.out_dtype, p.out_nchw, p.geglu = F32_T, F32_T, 0, 0
+    _lib.check(lib.sdk_conv_gemm_f32(C.byref(p), stream()))
+    torch.cuda.synchronize()
+    want = a.double() @ w.double().t()
+    if bias is not None:
+        want = want + bias.double()
+    e = rel_l2(out, want)
+    print(f"VAE attention fp32 {stage} S={S}: rel-L2 {e:.2e}")
+    assert e < 2e-5
+    if row0:
+        assert torch.isnan(out_all[:row0]).all(), "wrote outside the sample's rows"
