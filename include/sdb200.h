@@ -282,6 +282,20 @@ int sdk_linear_ln_info(void* handle, int* out, int n);          /* block_n, clus
 int sdk_linear_ln_launch(void* handle, void* stream);
 int sdk_linear_ln_destroy(void* handle);
 
+/* ---- LoRA merge into packed weights (the low-rank update W + up*down of a LoRA / LoCon adapter, merged at inference) -------------
+ *   dst[row_off + row_step*n][k] = cast( base[n][k] + sum_j up[n][j] * down[j][k] )      n < N, k < K
+ * base: fp32 [N][ld_base], the master weight in the packed k order (conv taps NHWC: [kh][kw][Cin]); up: fp32 [N][r] with the adapter
+ * scales folded in; down: fp32 [r][K]; several adapters on one target are concatenated along r.  r = 0 is a plain repack (up and
+ * down may be NULL).  fp32 FFMA, j in increasing order.  dst_dtype SDK_F32 | SDK_BF16 (round to nearest even).
+ * dst_layout SDK_LORA_ROW_MAJOR: dst is [dst_rows][K]; SDK_LORA_KBLOCK_MAJOR: dst is [K/64][dst_rows][64] (K % 64 == 0), the
+ * tensor-core weight layout (SdkTcGemmDesc.w_kmajor).  Not launched with programmatic dependent launch: kernels that follow it may
+ * read the weights it writes before their own griddepcontrol.wait (SdkTcGemmDesc.w_const).  SDK_ERR_ARG before any launch for
+ * NULL base / dst, non-positive sizes, ld_base < K, r < 0, missing factors, an unknown dtype or layout, or rows outside dst_rows. */
+#define SDK_LORA_ROW_MAJOR 0
+#define SDK_LORA_KBLOCK_MAJOR 1
+int sdk_lora_merge(const float* base, int64_t ld_base, const float* up, const float* down, int r, void* dst,
+                   int dst_dtype, int dst_layout, int dst_rows, int row_off, int row_step, int N, int K, void* stream);
+
 /* ---- plan-level entry: a program's LAUNCH LIST behind the C ABI, replayable, serialisable (engine file) -------------------------
  * The planning host records every launch of a program (one UNet forward = models/unet/unet.py:431-443, the context program, one
  * whole sampler step = the loop body of models/diffusion.py:223-236, a VAE decode, ...) with sdk_plan_add_launch; the plan ADOPTS the

@@ -81,6 +81,8 @@ SIGNATURES = {
     "sdk_linear_ln_info": [P, P, I32],
     "sdk_linear_ln_launch": [P, P],
     "sdk_linear_ln_destroy": [P],
+    # --- lora_merge.cu
+    "sdk_lora_merge": [P, I64, P, P, I32, P, I32, I32, I32, I32, I32, I32, I32, P],
     # --- plan.cu
     "sdk_plan_create": [P],
     "sdk_plan_destroy": [P],

@@ -82,7 +82,7 @@ const std::vector<FnEntry>& registry() {
         E(sdk_groupnorm_stats), E(sdk_groupnorm_apply), E(sdk_groupnorm_apply_cs), E(sdk_channel_stats), E(sdk_groupnorm_fused),
         E(sdk_groupnorm_cluster), E(sdk_layernorm), E(sdk_softmax_rows), E(sdk_embed_tokens), E(sdk_activation), E(sdk_cast_upsample),
         E(sdk_nchw_to_nhwc), E(sdk_time_sinusoid), E(sdk_gemv), E(sdk_conv_in), E(sdk_im2col_s2),
-        E(sdk_attention_f32), E(sdk_attention_f32_ex), E(sdk_attention_bf16),
+        E(sdk_attention_f32), E(sdk_attention_f32_ex), E(sdk_attention_bf16), E(sdk_lora_merge),
         entry("sdk_conv_gemm_f32", &sdk_conv_gemm_f32, FN_STRUCT),
         entry("sdk_tc_gemm_launch", &sdk_tc_gemm_launch, FN_HANDLE, H_TC_GEMM),
         entry("sdk_attention_tc_launch", &sdk_attention_tc_launch, FN_HANDLE, H_ATTENTION_TC),

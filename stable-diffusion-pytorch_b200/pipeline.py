@@ -59,6 +59,7 @@ class DenoiseLoop:
         self.hoist_time = True                                # precompute the time-embedding rows of the grid (exactly the per-step values)
         self._grid_key = None
         self._cond_ref, self._cond_version = None, -1
+        self._weights_version = pw.version
         self.launches_per_step = len(self.prog.body_ops) + 3
         self.inpaint_orig, self.inpaint_mask = None, None     # set_inpaint(): the step becomes the inpainting loop body
 
@@ -182,18 +183,26 @@ class DenoiseLoop:
             # time embedding -> 22 ResBlock projections depend only on t: run that chain once per grid point, keep the rows
             self.tb_table = None
             if self.hoist_time and p.nt == 1:
-                rows = []
-                for tv in self.ts_table.tolist():
-                    p.t_in.fill_(tv)
-                    p.launch(p.time_ops)
-                    rows.append(p.tb[0].clone())
-                self.tb_table = torch.stack(rows).contiguous()
-        if not same_context(context, self._cond_ref, self._cond_version):
+                with torch.inference_mode(False):                 # rewritten in place later, whatever mode that call runs in
+                    self.tb_table = torch.empty((len(self.ts_table), p.tb.shape[1]), dtype=torch.float32, device=self.device)
+                self._time_rows()
+        elif self.tb_table is not None and p.pw.version != self._weights_version:
+            self._time_rows()                                  # a LoRA merge changed tb.w: same tensor, the captured graph stays valid
+        if not same_context(context, self._cond_ref, self._cond_version) or p.pw.version != self._weights_version:
             if tuple(context.shape) != tuple(p.cond_in.shape):
                 raise RuntimeError(f"context shape {tuple(context.shape)} != {tuple(p.cond_in.shape)}")
             p.cond_in.copy_(context, non_blocking=True)
-            p.launch(p.ctx_ops)                                # cross-attention K/V once per generation (loop-invariant)
+            p.launch(p.ctx_ops)                                # cross-attention K/V once per generation and weights (loop-invariant)
             self._cond_ref, self._cond_version = context, tensor_version(context)
+        self._weights_version = p.pw.version
+
+    def _time_rows(self):
+        """tb_table[i] = the time-embedding projections at grid timestep i, written into the existing table."""
+        p = self.prog
+        for i, tv in enumerate(self.ts_table.tolist()):
+            p.t_in.fill_(tv)
+            p.launch(p.time_ops)
+            self.tb_table[i].copy_(p.tb[0])
 
     def step(self):
         """Advance the latent state by one sampler step (device-side timestep walk)."""

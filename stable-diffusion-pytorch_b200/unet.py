@@ -22,6 +22,7 @@ from typing import Dict, List, Optional, Union
 import torch
 
 from ._lib import BF16_T, F32_T
+from . import _lib, lora
 from .arch import BLOCK_OUT, Transformer, UNetArch, build_arch, param_spec
 from .program import _DT, GraphRunner, KernelWeights, LaunchProgram, ProgramModule
 
@@ -53,7 +54,12 @@ class PackedWeights(KernelWeights):
     attn2 k|v              -> one [2C][Dctx] matrix
     ffn.0.proj             -> rows interleaved (value_j, gate_j) so GEGLU fuses into the epilogue
     t_embed of all 22 ResBlocks -> one [sum Cout][1280] matrix (single batched mat-vec)
+
+    ``version`` counts the in-place LoRA merges into these tensors (UNet.load_lora): results cached from the weights -- the
+    cross-attention K/V of a context, the hoisted time projections of a sampling loop -- are recomputed when it changes.
     """
+
+    version = 0
 
     def _pack(self, net: "UNet"):
         a, sd, t, wdt, dev, conv_w = net.arch, self.sd, self.t, self.wdt, self.dev, self.conv_w
@@ -409,6 +415,7 @@ class UNet(ProgramModule):
         self.arch = build_arch(attention_head_dim, cross_attention_dim, in_channels, out_channels, block_out_channels,
                                down_block_types, t_embed_dim, num_attention_heads, eps)
         self._init_params(param_spec(self.arch))
+        self._lora: Dict[str, list] = {}       # adapter name -> [scale, {reference parameter name: lora.LoraModule}]
 
     # reference API no-ops (unet.py:404-428): inference path has no checkpointing; attention is always fused
     def gradient_checkpointing_enabled(self, enabled=False):
@@ -423,8 +430,81 @@ class UNet(ProgramModule):
         pw = self._packed.get(key)
         if pw is None:
             pw = PackedWeights(self, device, self.precision)
+            self._merge(pw, {ref for _, mods in self._lora.values() for ref in mods})
             self._packed[key] = pw
         return pw
+
+    # ---- LoRA adapters, merged into the packed weights in place ----------------------------------
+    @property
+    def lora_adapters(self) -> Dict[str, float]:
+        """{adapter name: scale} of the loaded adapters."""
+        return {n: s for n, (s, _) in self._lora.items()}
+
+    def load_lora(self, src, scale: float = 1.0, name: str = "default") -> List[str]:
+        """Merge a kohya or PEFT LoRA (``.safetensors`` path or state dict; LoCon convs included) into the packed weights as
+        ``scale * alpha / rank * up @ down``, replacing an adapter of the same name.  The parameters keep the base weights
+        (``state_dict()`` is unchanged); plans and captured graphs stay valid because the packed tensors are rewritten in place.
+        Returns the keys that are not for the UNet (text-encoder LoRA), which are not applied.  Raises ValueError naming the key
+        for a UNet key that does not fit, before anything changes."""
+        if self.ln_fold:
+            raise NotImplementedError("load_lora: the opt-in LayerNorm fold (SDB200_LN_FOLD=1) packs weights derived from the "
+                                      "LayerNorm parameters, which a merge does not rebuild")
+        mods, unapplied = lora.read_adapter(src, self.arch)
+        old = self._lora.get(name, [0.0, {}])[1]
+        self._lora[name] = [float(scale), mods]
+        self._remerge(set(old) | set(mods))
+        return unapplied
+
+    def set_lora_scale(self, name: str, scale: float):
+        """Change the scale of a loaded adapter and re-merge the targets it touches."""
+        if name not in self._lora:
+            raise KeyError(f"no LoRA adapter named {name!r} (loaded: {sorted(self._lora)})")
+        self._lora[name][0] = float(scale)
+        self._remerge(set(self._lora[name][1]))
+
+    def unload_lora(self, name: Optional[str] = None):
+        """Remove one adapter (or all, ``name=None``): the targets are rebuilt from the base weights, bit for bit."""
+        names = list(self._lora) if name is None else [name]
+        refs = set()
+        for n in names:
+            if n not in self._lora:
+                raise KeyError(f"no LoRA adapter named {n!r} (loaded: {sorted(self._lora)})")
+            refs |= set(self._lora.pop(n)[1])
+        self._remerge(refs)
+
+    def _remerge(self, refs):
+        for pw in self._packed.values():
+            self._merge(pw, refs)
+
+    def _merge(self, pw: PackedWeights, refs):
+        """Rebuild every packed tensor of the parameters ``refs`` from the fp32 master and the adapters with a non-zero scale, in
+        adapter-name order (so the result does not depend on the order of the calls)."""
+        if not refs:
+            return
+        lib = _lib.lib()
+        params = dict(self.named_parameters())
+        with torch.inference_mode(False), torch.no_grad(), torch.cuda.device(pw.device):
+            # an fp32 pack on the parameters' device shares the storage of the weights it did not have to transform: give such a
+            # parameter its own copy, so that merges into the pack never change the master weights
+            shared = {p.untyped_storage().data_ptr(): p for p in params.values()}
+            for t in pw.t.values():
+                p = shared.pop(t.untyped_storage().data_ptr(), None)
+                if p is not None:
+                    p.data = p.data.clone()
+            stream = torch.cuda.current_stream(pw.device).cuda_stream
+            for ref in sorted(refs):
+                mods = [(m[ref], s) for _, (s, m) in sorted(self._lora.items()) if ref in m and s != 0.0]
+                for op in lora.merge_ops(self.arch, pw, ref, params[ref], mods):
+                    dst, up, down = op["dst"], op["up"], op["down"]
+                    r = 0 if up is None else up.shape[1]
+                    n, k = op["base"].shape
+                    # not a PDL launch (lora_merge.cu): kernels of this stream read packed weights before their own grid-dependency
+                    # wait, so the next launch must start after the merge has completed
+                    code = BF16_T if dst.dtype == torch.bfloat16 else F32_T
+                    _lib.check(lib.sdk_lora_merge(op["base"].data_ptr(), k, 0 if up is None else up.data_ptr(),
+                                                  0 if down is None else down.data_ptr(), r, dst.data_ptr() + op["offset"] * dst.element_size(),
+                                                  code, op["layout"], op["dst_rows"], op["row_off"], op["row_step"], n, k, stream))
+        pw.version += 1
 
     def forward(self, x: torch.Tensor, timestep: torch.LongTensor, cond: torch.Tensor) -> torch.Tensor:
         """reference: unet.py:431-443.  x (B,C,h,w) NCHW float; timestep int64 (1,) or (B,); cond (B|1,Sk,Dctx)."""
@@ -495,14 +575,16 @@ class _Runner(GraphRunner):
         super().__init__(prog, use_graph)
         self._cond_ref = None
         self._cond_version = -1
+        self._weights_version = prog.pw.version
 
     def __call__(self, x, timestep, cond):
         p = self.prog
         p.x_in.copy_(x, non_blocking=True)
         p.t_in.copy_(timestep.to(torch.int64), non_blocking=True)
-        if not same_context(cond, self._cond_ref, self._cond_version):
+        if not same_context(cond, self._cond_ref, self._cond_version) or p.pw.version != self._weights_version:
             p.cond_in.copy_(cond, non_blocking=True)
-            p.launch(p.ctx_ops)                       # cross-attention K/V: once per context, not per step
+            p.launch(p.ctx_ops)                       # cross-attention K/V: once per context and weights, not per step
             self._cond_ref, self._cond_version = cond, tensor_version(cond)
+            self._weights_version = p.pw.version
         self.run()
         return p.out.clone()
